@@ -13,7 +13,10 @@ fp16 matcher operands), the mode that passes the parity gates of SURVEY.md 8d; t
 'fast' mode beside it (`fast_mode`), an encoder roofline (`encoder`), and a fixed-size strong-scaling leg (`strong`: 4096 x 4096
 pairs row-sharded over the N ranks INCLUDING the all-gather of the score rows).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode parity_tc|fast|parity]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode parity_tc|fast|parity] [--dump-outputs DIR]
+
+--dump-outputs DIR writes the score rows the timed path returned in its last step, one file per rank, so that two builds can
+be compared output for output on identical seeded inputs.
 """
 import argparse
 import glob
@@ -58,6 +61,7 @@ MODE_TEXT = {
                  "cn_linear_tma.cu), logits within 1e-4 of the reference",
 }
 DTYPE = {"parity_tc": "f16", "fast": "bf16", "parity": "f32", "parity_x3": "tf32x3"}
+DUMP_BYTES = 64 * 10**6          # --dump-outputs: at most this many bytes over all files of all ranks
 
 
 def peaks():
@@ -183,6 +187,46 @@ def parity_block(model, dev, rows=384, cols=256):
             "embedding_max_abs": float((ht.cpu() - oht).abs().max()), "oracle_cpu_s": cpu_s}
 
 
+def dump_scores(out_dir, rows, rank, world):
+    """this rank's (T_r, D) score rows as out_dir/scores_rank<r>.npy (float32).  When they exceed the rank's share of DUMP_BYTES,
+    a fixed, seeded sample of rows is written instead, with the sampled row indices in scores_rank<r>_rows.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    s = rows.float().cpu()
+    path = os.path.join(out_dir, f"scores_rank{rank}")
+    keep = (DUMP_BYTES // world - 2 * 128) // (4 * s.shape[1] + 8)          # 128: an .npy header
+    if s.shape[0] > keep:
+        idx = torch.randperm(s.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        s = s[idx]
+        np.save(path + "_rows.npy", idx.double().numpy())
+    np.save(path + ".npy", s.numpy())
+
+
+def bench_model(cfg, mode, dev):
+    """the benchmarked model: configuration `cfg` (a CONFIGS entry) with its default init under seed 66, in `mode`"""
+    from pcreid_b200 import synthetic as S
+    n = cfg["npts"]
+    torch.manual_seed(66)
+    from pcreid_b200.models import build_model
+    model = build_model({"pt": S.point_transformer_cfg, "dgcnn": S.dgcnn_cfg}[cfg["kind"]]((n, n // 2, n // 4))).eval().to(dev)
+    model.set_mode(mode)
+    return model
+
+
+def bench_inputs(npts, tracks, dets, rank=0, world=1, strong=False):
+    """this rank's host (tracks, detections), seeded synthetic objects: its share of `tracks` rows (strong scaling, seed 1000) or
+    `tracks` rows of its own (weak scaling, seed 1000 + rank), and its share of the `dets` detections (seed 1)"""
+    from pcreid_b200 import synthetic as S
+    from pcreid_b200.parallel import shard_range
+    if strong:
+        t0, t1 = shard_range(tracks, rank, world)
+        t = S.synth_objects(tracks, npts, 1000)[t0:t1].contiguous()
+    else:
+        t = S.synth_objects(tracks, npts, 1000 + rank)
+    d0, d1 = shard_range(dets, rank, world)
+    return t, S.synth_objects(dets, npts, 1)[d0:d1].contiguous()
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -216,7 +260,13 @@ def main():
     ap.add_argument("--dets", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU legs (cpu_baseline, parity)")
     ap.add_argument("--no-extra", action="store_true", help="skip the fast-mode and strong-scaling legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the score rows of the last timed step to DIR/scores_rank<r>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the CUDA path's scores: it needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -247,13 +297,8 @@ def main():
     d0, d1 = shard_range(D, rank, world)
     det_counts = [shard_range(D, r, world)[1] - shard_range(D, r, world)[0] for r in range(world)]
 
-    torch.manual_seed(66)
-    from pcreid_b200.models import build_model
-    model_cfg = {"pt": S.point_transformer_cfg, "dgcnn": S.dgcnn_cfg}[cfg["kind"]](BLIST)
-    model = build_model(model_cfg).eval().to(dev)
-    model.set_mode(args.mode)
-    tracks_h = (S.synth_objects(T_total, NPTS, 1000)[t0_:t1_].contiguous() if strong_main else S.synth_objects(T_loc, NPTS, 1000 + rank)).pin_memory()
-    dets_h = S.synth_objects(D, NPTS, 1)[d0:d1].contiguous().pin_memory()
+    model = bench_model(cfg, args.mode, dev)
+    tracks_h, dets_h = (x.pin_memory() for x in bench_inputs(NPTS, T_arg, D, rank, world, strong_main))
     tracks_d, dets_d = tracks_h.to(dev), dets_h.to(dev)
     out_h = torch.empty((T_loc, D), dtype=torch.float32).pin_memory()
 
@@ -273,18 +318,19 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """-> (total ms, per-step ms, what fn returned in the last step)"""
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(steps + 1)]
         barrier()
         ev[0].record()
         for i in range(steps):
-            fn()
+            out = fn()
             ev[i + 1].record()
         barrier()
         ms = ev[0].elapsed_time(ev[steps])
         t = torch.tensor([ms], device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item()), [ev[i].elapsed_time(ev[i + 1]) for i in range(steps)]
+        return float(t.item()), [ev[i].elapsed_time(ev[i + 1]) for i in range(steps)], out
 
     for _ in range(args.warmup):
         step_device()
@@ -292,9 +338,12 @@ def main():
     if rank == 0:
         sampler.start()
     calls0 = _lib.ABI_CALLS
-    total_ms, per_step = timed(step_device, args.steps)
+    total_ms, per_step, rows = timed(step_device, args.steps)
     launches = _lib.ABI_CALLS - calls0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_scores(args.dump_outputs, rows, rank, world)
+    del rows
     # phase split (device events, extra steps): encode vs match.  Inside the timed steps the ~90 launches of an encoder pass are
     # issued while the previous step's match still runs; measured alone after a synchronize they would be bound by the host's
     # launch rate, so the encode phase is timed as the public API's CUDA-graph replay (ReIDNet.enable_cuda_graphs): device time.
@@ -322,7 +371,7 @@ def main():
     del xt, ht, xd, hd
     for _ in range(1):
         step_e2e()
-    e2e_ms, _ = timed(step_e2e, args.steps)
+    e2e_ms, _, _ = timed(step_e2e, args.steps)
     # encode phase (after every headline number has been taken: the capture owns a private memory pool)
     model.enable_cuda_graphs(True)
     encode_and_gather(model, tracks_d, dets_d, det_counts)          # capture
@@ -340,7 +389,7 @@ def main():
         model.set_mode("fast")
         for _ in range(2):
             step_device()
-        f_ms, _ = timed(step_device, min(args.steps, 5))
+        f_ms, _, _ = timed(step_device, min(args.steps, 5))
         fast = {"value": T_total * D / (f_ms / min(args.steps, 5) * 1e-3), "unit": "pairs/s", "ms_per_step": f_ms / min(args.steps, 5),
                 "dtype": "bf16", "mode": MODE_TEXT["fast"]}
         model.set_mode(args.mode)
@@ -361,7 +410,7 @@ def main():
 
         step_strong()
         n_s = 2
-        s_ms, _ = timed(step_strong, n_s)
+        s_ms, _, _ = timed(step_strong, n_s)
         gb = gathered_bytes(model, NPTS, s_dc, s_tc, gather_scores=True)
         strong = {"workload": f"fixed {Ts}x{Ds} all-pairs xcorr_eff @ {NPTS} pts + encode of {Ts}+{Ds} objects, track rows and detections "
                               f"sharded over {world} rank(s); timed region includes the all-gather of the detection embeddings (overlapped "

@@ -7,7 +7,7 @@ Follows, line by line:
   mmdet3d/core/bbox/structures/depth_box3d.py:256-282   depth -> LiDAR frame for points and boxes
   mmdet3d/core/bbox/structures/box_3d_mode.py:125-148   DEPTH -> LIDAR box conversion (rt_mat, size swap)
   mmdet3d/ops/roiaware_pool3d/src/points_in_boxes_cuda.cu:24-49, 79-105   the in-box test
-PINNED (tests/test_frontend_pinned.py, wherever /root/reference exists) against the reference's own pc_utils.py and
+PINNED (tests/test_frontend_pinned.py, wherever PCREID_REFERENCE_ROOT names the upstream source tree) against the reference's own pc_utils.py and
 core/bbox/structures/*.py imported unmodified by path (oracle/ref_loader.load_frontend): box origin / frame conversion and
 crop order exactly, centred coordinates within 2e-5 (fp32 torch there, fp64 numpy here), sampling with the same torch.randint
 draws.  Stand-ins there: pytorch3d (absent; Pointclouds.points_padded and axis_angle_to_matrix restated from pytorch3d 0.7)

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.npz by running the UNMODIFIED reference modules
-(imported by path from /root/reference through oracle/ref_loader.py) on seeded synthetic inputs.
+(imported by path from $PCREID_REFERENCE_ROOT through oracle/ref_loader.py) on seeded synthetic inputs.
 
-    python oracle/make_golden.py          # only works where /root/reference exists
+    python oracle/make_golden.py          # needs PCREID_REFERENCE_ROOT=<upstream source tree>
 
 The reference ships no golden vectors (SURVEY.md section 4); these fixtures are what pins the oracle and
 the CUDA path on machines where the reference tree is absent (the GPU box).  Weights are the reference

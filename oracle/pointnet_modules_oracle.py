@@ -2,7 +2,7 @@
 (mmdet3d/ops/pointnet_modules/point_sa_module.py:164-208 BasePointSAModule.forward, point_fp_module.py:39-79
 PointFPModule.forward) as plain torch over the op oracle (oracle/ops_oracle.py).
 
-PINNED (tests/test_pointnet_modules_pinned.py, wherever /root/reference exists): bit-exact against the reference's own module
+PINNED (tests/test_pointnet_modules_pinned.py, wherever PCREID_REFERENCE_ROOT names the upstream source tree): bit-exact against the reference's own module
 files imported unmodified by path (oracle/ref_loader.load_pointnet_modules) -- BasePointSAModule / PointSAModuleMSG /
 PointSAModule / build_sa_module, PointFPModule, QueryAndGroup / GroupAll, Points_Sampler / calc_square_dist -- run on CPU with
 (a) the compiled CUDA ops replaced by oracle/ops_oracle.py, which is pinned to the reference .cu files on the GPU box, and

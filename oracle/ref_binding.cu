@@ -1,6 +1,6 @@
 // TEST INFRASTRUCTURE ONLY -- C-ABI shim over the reference's own CUDA launchers.
 // oracle/Makefile compiles the reference .cu files UNMODIFIED, from where they lie under
-// /root/reference/mmdet3d/ops/*/src/, together with this file into oracle/_ref/libref_ops.so.
+// $PCREID_REFERENCE_ROOT/mmdet3d/ops/*/src/, together with this file into oracle/_ref/libref_ops.so.
 // (The reference's pybind .cpp wrappers include the removed THC/THC.h and do not build against
 // torch 2.11, so the launchers are bound directly.)  Gives a bit-level GPU oracle and the
 // "reference kernel recompiled for sm_100a" speed bar on the GPU box.

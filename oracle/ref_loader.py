@@ -1,6 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- loads the *unmodified* reference leaf modules by path.
 
-Only usable where ``/root/reference`` exists (the build container).  It is used to
+Only usable where a checkout of the upstream project (bentherien/point-cloud-reid) is named by the environment variable
+``PCREID_REFERENCE_ROOT``; the repository does not contain it.  It is used to
   (1) pin ``oracle/reid_oracle.py`` (our CPU restatement) against the real reference code, and
   (2) generate the committed golden vectors under ``tests/golden/`` (``oracle/make_golden.py``).
 Nothing in the product package, ``bench.py`` or the ``-m gpu`` tests may import this file.
@@ -21,13 +22,14 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("PCREID_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("PCREID_REFERENCE_ROOT", "")
+MISSING = "needs the upstream point-cloud-reid source tree, named by PCREID_REFERENCE_ROOT (not part of this repository)"
 _MODELS = os.path.join(REF_ROOT, "mmdet3d", "models")
 _PKG = "_pcreid_ref_models"
 
 
 def available():
-    return os.path.isdir(_MODELS)
+    return bool(REF_ROOT) and os.path.isdir(_MODELS)
 
 
 class _TorchProxy(types.ModuleType):
@@ -61,7 +63,7 @@ def _load(name):
 def load():
     """Returns a namespace with the reference classes used on the hot path."""
     if not available():
-        raise RuntimeError(f"reference tree not found at {REF_ROOT}")
+        raise RuntimeError(f"reference tree not found: PCREID_REFERENCE_ROOT={REF_ROOT!r}")
     import fractions
     if not hasattr(fractions, "gcd"):
         fractions.gcd = math.gcd
@@ -96,7 +98,7 @@ _OPS_PKG = "_pcreid_ref_ops"
 
 
 def pointnet_modules_available():
-    return os.path.isdir(os.path.join(_OPS, "pointnet_modules"))
+    return bool(REF_ROOT) and os.path.isdir(os.path.join(_OPS, "pointnet_modules"))
 
 
 def load_pointnet_modules():
@@ -251,7 +253,7 @@ _PC_UTILS = os.path.join(_MODELS, "trackers", "deprecated", "pc_utils.py")
 
 
 def frontend_available():
-    return os.path.isdir(_STRUCTS) and os.path.exists(_PC_UTILS)
+    return bool(REF_ROOT) and os.path.isdir(_STRUCTS) and os.path.exists(_PC_UTILS)
 
 
 def load_frontend():
@@ -359,7 +361,7 @@ _TRK = os.path.join(_MODELS, "trackers", "deprecated")
 
 
 def tracker_available():
-    return os.path.exists(os.path.join(_TRK, "tracking_point_reid.py")) and os.path.exists(os.path.join(_TRK, "tracking_feature_set.py"))
+    return bool(REF_ROOT) and os.path.exists(os.path.join(_TRK, "tracking_point_reid.py")) and os.path.exists(os.path.join(_TRK, "tracking_feature_set.py"))
 
 
 def load_tracker():

@@ -7,6 +7,8 @@ import sys
 
 import glob
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -53,3 +55,47 @@ def test_reference_arm_prints_one_contract_line():
     assert d["cpu_baseline"]["value"] == d["value"] and d["cpu_baseline"]["cores"] >= 1
     ours = _latest_bench_line()
     assert d["metric"] == ours["metric"] and d["unit"] == ours["unit"]
+
+
+def test_dump_outputs_samples_rows_beyond_the_budget(tmp_path, monkeypatch):
+    """score rows over a rank's share of the byte budget are cut to the same seeded row sample on every run"""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    budget = 2 * (10 * (4 * 32 + 8) + 2 * 128)          # two ranks, room for ten rows and two .npy headers each
+    monkeypatch.setattr(bench, "DUMP_BYTES", budget)
+    rows = torch.arange(100 * 32, dtype=torch.float32).reshape(100, 32)
+    for run in ("a", "b"):
+        bench.dump_scores(str(tmp_path / run), rows, 1, 2)
+    idx = np.load(tmp_path / "a" / "scores_rank1_rows.npy")
+    s = np.load(tmp_path / "a" / "scores_rank1.npy")
+    assert idx.dtype == np.float64 and idx.shape == (10,) and (np.diff(idx) > 0).all()
+    assert s.dtype == np.float32 and np.array_equal(s, rows.numpy()[idx.astype(np.int64)])
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "scores_rank1_rows.npy"))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= budget // 2
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_steps_scores(tmp_path):
+    """--dump-outputs writes the score rows the timed path returned, and they are what the public API computes on the same seeded
+    inputs in another process; --steps sets the number of timed steps"""
+    import numpy as np
+    from pcreid_b200.parallel import match_all_pairs_sharded
+    sys.path.insert(0, ROOT)
+    import bench
+    T, D = 64, 48
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "1", "--tracks", str(T),
+                          "--dets", str(D), "--no-cpu-baseline", "--no-extra", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == 3 and len(line["per_step_ms"]) == 3
+    assert sorted(os.listdir(tmp_path)) == ["scores_rank0.npy"]
+    got = np.load(tmp_path / "scores_rank0.npy")
+    assert got.dtype == np.float32 and got.shape == (T, D) and np.isfinite(got).all()
+    cfg = bench.CONFIGS["c2"]                  # bench.py's defaults: the headline configuration and mode
+    model = bench.bench_model(cfg, "parity_tc", "cuda")
+    t, d = bench.bench_inputs(cfg["npts"], T, D)
+    rows = match_all_pairs_sharded(model, t.cuda(), d.cuda(), [D])
+    assert np.array_equal(got, rows.cpu().numpy())

@@ -1,7 +1,7 @@
 """Pins oracle/frontend_oracle.py (crop -> centre -> resample, SURVEY 8f row 2) to the reference's OWN code:
 models/trackers/deprecated/pc_utils.py (interpolate_per_frame, get_input_batch) and core/bbox/structures/*.py
 (DepthInstance3DBoxes, Box3DMode.convert) imported unmodified by path (oracle/ref_loader.load_frontend) and run on CPU; pytorch3d
-and the compiled points_in_boxes op are stand-ins (see the loader).  Runs where /root/reference exists."""
+and the compiled points_in_boxes op are stand-ins (see the loader).  Runs where PCREID_REFERENCE_ROOT names the upstream source tree."""
 import numpy as np
 import pytest
 import torch
@@ -9,7 +9,7 @@ import torch
 from oracle import frontend_oracle as FO
 from oracle import ref_loader
 
-pytestmark = pytest.mark.skipif(not ref_loader.frontend_available(), reason="reference tree not present on this machine")
+pytestmark = pytest.mark.skipif(not ref_loader.frontend_available(), reason=ref_loader.MISSING)
 
 
 @pytest.fixture(scope="module")

@@ -1,5 +1,5 @@
 """Pins the oracle (oracle/reid_oracle.py): (1) bit-exact against the unmodified reference modules where
-/root/reference exists, (2) against the committed golden vectors everywhere."""
+PCREID_REFERENCE_ROOT names the upstream source tree, (2) against the committed golden vectors everywhere."""
 import numpy as np
 import pytest
 import torch
@@ -7,7 +7,7 @@ import torch
 import helpers
 from oracle import ref_loader, reid_oracle as O
 
-needs_ref = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present on this machine")
+needs_ref = pytest.mark.skipif(not ref_loader.available(), reason=ref_loader.MISSING)
 
 
 def _load_ref_sd(mod, prefix, sd):

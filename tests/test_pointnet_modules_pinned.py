@@ -2,14 +2,14 @@
 against) to the reference's OWN module code: ops/pointnet_modules/{point_sa_module,point_fp_module,builder}.py,
 ops/group_points/group_points.py and ops/furthest_point_sample/{points_sampler,utils}.py are imported unmodified by path
 (oracle/ref_loader.load_pointnet_modules) and run on CPU, with the compiled CUDA ops replaced by the op oracle (itself pinned
-to the reference .cu files on the GPU box) and mmcv's ConvModule by a torch stand-in.  Runs where /root/reference exists."""
+to the reference .cu files on the GPU box) and mmcv's ConvModule by a torch stand-in.  Runs where PCREID_REFERENCE_ROOT names the upstream source tree."""
 import pytest
 import torch
 
 from oracle import pointnet_modules_oracle as PO
 from oracle import ref_loader, reid_oracle as O
 
-pytestmark = pytest.mark.skipif(not ref_loader.pointnet_modules_available(), reason="reference tree not present on this machine")
+pytestmark = pytest.mark.skipif(not ref_loader.pointnet_modules_available(), reason=ref_loader.MISSING)
 
 
 def _randomise_bn(m, seed):

@@ -7,7 +7,7 @@ mmdet's BaseDetector base class and pytorch3d's training-only chamfer loss) and 
     match_forward_inference, forward_test);
   * the product's modules (with the kernel *specification* emulation of tests/fake_kernels.py on CPU) return the same result
     dict as the real forward_test, key for key, and load the real class's state_dict with strict=True.
-Runs where /root/reference exists."""
+Runs where PCREID_REFERENCE_ROOT names the upstream source tree."""
 import copy
 
 import pytest
@@ -17,7 +17,7 @@ import fake_kernels
 import helpers
 from oracle import ref_loader, reid_oracle as O
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present on this machine")
+pytestmark = pytest.mark.skipif(not ref_loader.available(), reason=ref_loader.MISSING)
 
 SHIPPED = dict(losses_to_use=dict(kl=False, match=True, cls=False, shape=False, fp=False, triplet=False),
                alpha=dict(kl=1, match=1, cls=1, shape=1, fp=1, vis=1, triplet=1), triplet_loss=dict(margin=10, p=2),

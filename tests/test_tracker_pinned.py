@@ -6,7 +6,7 @@ import torch
 
 from oracle import ref_loader, reid_oracle as O
 
-pytestmark = pytest.mark.skipif(not ref_loader.tracker_available(), reason="reference tree not present on this machine")
+pytestmark = pytest.mark.skipif(not ref_loader.tracker_available(), reason=ref_loader.MISSING)
 
 
 @pytest.fixture(scope="module")

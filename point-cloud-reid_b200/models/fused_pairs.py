@@ -7,6 +7,11 @@ modes of ReIDNet.match_all_pairs / match_forward_inference:
               LayerNorm outputs, elu+1 features, projections of those, and key/value sums that are stored divided by the
               point count (the attention read-out is a ratio, so the scale cancels; LinearAttention's eps is scaled
               with it).  Conversions saturate instead of overflowing.
+              Feature range: tests/test_gpu_fused_phases.py sweeps the search / template features h from 1/16 to 16 times
+              the encoder's scale (max|h| ~ 2): both modes stay inside their gates (parity_tc |dlogit| 3.1e-3, fast 1.1e-2 at
+              x16 on an NVIDIA B200).  The largest fp16 operand grows as the square of that scale (the unnormalised
+              key/value products of the stage-1 attention operand, max ~ 0.75 at x1), so fp16 saturation is estimated to begin
+              near x300 (not exercised by the tests).
 
 Everything that depends on one object only is computed once per object with the fp32 kernels and packed to 16-bit
 operand images (stage-1 queries elu(Wq1 h)+1, h + beta2, Wv2 pos2(xyz), and the stage-1 attention operand

@@ -64,10 +64,10 @@ def test_fused_symmetry_and_determinism(mode):
 
 
 @pytest.mark.parametrize("mode", ["fast", "parity_tc"])
-@pytest.mark.parametrize("N", [256, 128])
+@pytest.mark.parametrize("N", [256, 128, 1024])
 def test_full_tensor_core_mode_end_to_end(N, mode):
     """set_mode('fast' | 'parity_tc'): tf32 tensor-core SA MLPs / attention blocks in the encoder + fused bf16 / fp16 matcher,
-    against the oracle end to end."""
+    against the oracle end to end; N = 1024 is the Waymo config (C4, backbone_list (1024, 512, 256), 8 tiles per object)."""
     m, orc = helpers.build_pair("pt", (N, N // 2, N // 4), device=DEV)
     m.set_mode(mode)
     t, d = O.synth_objects(6, N, 10), O.synth_objects(5, N, 11)
@@ -108,32 +108,44 @@ def test_concat_head_tensor_core_matches_parity_and_oracle(T, D, masked):
         assert ok, f"top-1 changed on a decisive row (agreement {agree}, {n} decisive rows)"
 
 
+# raw top-1 agreement of the 64 x 64 oracle block (one flip costs 1/64); measured on an NVIDIA B200 (1000 W power limit):
+# fast 62/64 = 0.969 (|dlogit| 9.6e-3), parity_tc 63/64 = 0.984 (|dlogit| 1.2e-3) -- two more flips allowed in parity_tc, four in fast
+TOP1_MIN = {"fast": 0.9, "parity_tc": 0.95}
+
+
 def test_full_size_config_properties():
-    """BASELINE configs[1] at its full size (1024 tracks x 1024 detections x 256 points, fast mode): size-independent
-    properties instead of an oracle pass -- (1) the dense row-chunked driver and the pair-list driver give the same logit for
-    the same pair, (2) scoring a row block on its own equals the rows of the full matrix (what the row-sharded multi-GPU
-    driver relies on), (3) swapping the roles of the two sets transposes the matrix (xcorr_eff + 'both' pooling is symmetric),
-    (4) a sampled 6 x 6 block agrees with the oracle within the fast-mode tolerance."""
+    """BASELINE configs[1] at its full size (1024 tracks x 1024 detections x 256 points), in both tensor-core modes:
+    (1) the dense row-chunked driver and the pair-list driver give the same logit for the same pair, (2) scoring a row block on
+    its own equals the rows of the full matrix (what the row-sharded multi-GPU driver relies on), (3) swapping the roles of the two
+    sets transposes the matrix (xcorr_eff + 'both' pooling is symmetric), (4) a sampled 64 x 64 block agrees with the oracle within
+    the mode's gate, keeps the top-1 decision on every decisive row and agrees on the raw top-1 of at least TOP1_MIN of its rows."""
     T = D = 1024
     m, orc = helpers.build_pair("pt", (256, 128, 64), device=DEV, perturb=False)
-    m.set_mode('fast')
     t, d = O.synth_objects(T, 256, 0), O.synth_objects(D, 256, 1)
-    xt, ht = m.encode(t.to(DEV))
-    xd, hd = m.encode(d.to(DEV))
-    L = m.match_all_pairs(ht, xt, hd, xd)
-    assert L.shape == (T, D) and torch.isfinite(L).all()
-    mask = torch.rand(T, D, generator=torch.Generator().manual_seed(1)) < 2e-3
-    Lm = m.match_all_pairs(ht, xt, hd, xd, pair_mask=mask.to(DEV))
-    assert int(mask.sum()) > 1000 and torch.equal(Lm[mask.to(DEV)], L[mask.to(DEV)]) and (Lm[~mask.to(DEV)] == 0).all()
-    rows = slice(384, 512)
-    assert torch.equal(m.match_all_pairs(ht[rows], xt[rows], hd, xd), L[rows])
-    Lt = m.match_all_pairs(hd[:256], xd[:256], ht[:256], xt[:256])
-    assert (Lt - L[:256, :256].t()).abs().max() < TOL_FAST
-    ti, di = torch.tensor([0, 1, 511, 512, 1022, 1023]), torch.tensor([3, 64, 65, 700, 1000, 1023])
+    g = torch.Generator().manual_seed(2)
+    ti, di = torch.randperm(T, generator=g)[:64].sort()[0], torch.randperm(D, generator=g)[:64].sort()[0]
     oxt, oht = orc.encode(t[ti])
     oxd, ohd = orc.encode(d[di])
     Lo = orc.match_all_pairs(oht, oxt, ohd, oxd)
-    assert (L[ti][:, di].cpu() - Lo).abs().max() < TOL_FAST
+    mask = torch.rand(T, D, generator=torch.Generator().manual_seed(1)) < 2e-3
+    for mode in ("fast", "parity_tc"):
+        m.set_mode(mode)
+        xt, ht = m.encode(t.to(DEV))
+        xd, hd = m.encode(d.to(DEV))
+        L = m.match_all_pairs(ht, xt, hd, xd)
+        assert L.shape == (T, D) and torch.isfinite(L).all()
+        Lm = m.match_all_pairs(ht, xt, hd, xd, pair_mask=mask.to(DEV))
+        assert int(mask.sum()) > 1000 and torch.equal(Lm[mask.to(DEV)], L[mask.to(DEV)]) and (Lm[~mask.to(DEV)] == 0).all()
+        rows = slice(384, 512)
+        assert torch.equal(m.match_all_pairs(ht[rows], xt[rows], hd, xd), L[rows])
+        Lt = m.match_all_pairs(hd[:256], xd[:256], ht[:256], xt[:256])
+        assert (Lt - L[:256, :256].t()).abs().max() < TOL[mode]
+        Lb = L[ti][:, di].cpu()
+        err = (Lb - Lo).abs().max().item()
+        assert err < TOL[mode], f"{mode}-mode logits off the oracle by {err}"
+        ok, agree, n = helpers.margin_aware_top1(Lo, Lb, err)
+        assert ok, f"{mode}: top-1 changed on a decisive row (agreement {agree}, {n} decisive rows)"
+        assert agree >= TOP1_MIN[mode], f"{mode}: raw top-1 agreement {agree}"
 
 
 @pytest.mark.parametrize("mode", ["fast", "parity_tc"])

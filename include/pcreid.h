@@ -252,6 +252,18 @@ int pcreid_pair_concat_head(int T, int D, int E, int G, const float* A, const fl
                             const float* W2, const float* g1, const float* be1, const float* g2, const float* be2,
                             const float* w, float b0, const unsigned char* mask, float* out, void* stream);
 
+/* Gated linear assignment of tracks to detections (csrc/assign.cu), the association step after the (T, D) logits: B problems
+ * of score (B, T, D) f32 (higher = more alike), mask (B, T, D) u8 or NULL (all admissible), threshold min_score.  A pair is
+ * admissible when mask != 0, the score is finite and score > min_score; its weight is double(score) - double(min_score).
+ * Each problem gets a matching of admissible pairs of maximum total weight (each track and detection at most once):
+ * det_for_track (B, T) / track_for_det (B, D) int32, -1 = unmatched.  Among several optimal matchings the choice is
+ * deterministic and per problem (independent of the other problems of the call).  One CTA per problem: shortest augmenting
+ * paths (Jonker-Volgenant / Crouse) with float64 duals.  work: B * pcreid_lsap_workspace_bytes(T, D) bytes of device scratch.
+ * 0 <= T, D <= 4096 and B <= 65535, else PCREID_ERR_UNSUPPORTED; a non-finite min_score is PCREID_ERR_ARG. */
+int pcreid_lsap_workspace_bytes(int T, int D);   /* per problem; -1 outside the supported shapes */
+int pcreid_lsap(int B, int T, int D, const float* score, const unsigned char* mask, float min_score, int* det_for_track,
+                int* track_for_det, void* work, void* stream);
+
 /* ------------------------------------------------------------------ B'. fused tensor-core match path --- */
 /* Tensor-core modes of the xcorr_eff head (csrc/pair_tc.cu, csrc/pair_tc2.cu): tcgen05 kind::f16 GEMMs with fp32
  * accumulation and fp32 norms.  `fmt` selects the 16-bit operand format of EVERY operand image of a call chain:

@@ -97,6 +97,8 @@ _SIGS = {
     "pcreid_sa_edge_mlp_tc2": [c_int, c_int, c_int, c_int, c_int] + [c_vp] * 8 + [c_int, c_int, c_vp],
     "pcreid_pair_concat_head_tc": [c_int, c_int, c_int, c_int] + [c_vp] * 10 + [c_float, c_vp, c_vp, c_int, c_vp],
     "pcreid_pair_concat_head": [c_int, c_int, c_int, c_int] + [c_vp] * 10 + [c_float, c_vp, c_vp, c_vp],
+    "pcreid_lsap_workspace_bytes": [c_int, c_int],
+    "pcreid_lsap": [c_int, c_int, c_int, c_vp, c_vp, c_float, c_vp, c_vp, c_vp, c_vp],
 }
 
 ERRORS = {1: "PCREID_ERR_ARG (bad pointer/size)", 2: "PCREID_ERR_LAUNCH (CUDA launch failed)",

@@ -5,6 +5,7 @@ Feature tensors are channel-major ``(B, C, N)`` (the reference's layout) with un
 arbitrary object / channel strides are passed through, so views such as ``qkv[:, :C]`` cost nothing.
 """
 import ctypes
+import math
 
 import torch
 
@@ -535,6 +536,48 @@ def pair_concat_head(a, bv, et, ed, w2, g1, be1, g2, be2, w, b0, groups, mask=No
     out = torch.empty((T, D), device=a.device, dtype=torch.float32)
     _OPS.pair_concat_head(T, D, E, groups, a, bv, et, ed, w2, g1, be1, g2, be2, w, float(b0), mask, out)
     return out
+
+
+LSAP_MAX_SIZE, LSAP_MAX_BATCH = 4096, 65535
+
+
+def linear_assignment(score, min_score, pair_mask=None):
+    """Maximum-weight matching of tracks to detections (pcreid_lsap).  score (T, D) or (B, T, D) CUDA float32, higher = more
+    alike (the logits of match_all_pairs); pair_mask bool of the same shape or None (e.g. class_gate).  A pair may be matched
+    only when pair_mask allows it, its score is finite and score > min_score; the matching maximises the sum of
+    score - min_score (float64).  -> (det_for_track (..., T), track_for_det (..., D)) int64 on the device, -1 = unmatched.
+    Checks shapes only: no host synchronisation, so the call can be captured in a CUDA graph."""
+    _need_cuda(score, pair_mask)
+    if score.dtype != torch.float32:
+        raise TypeError("score must be float32")
+    if score.dim() not in (2, 3):
+        raise ValueError(f"score must be (T, D) or (B, T, D); got {tuple(score.shape)}")
+    if isinstance(min_score, torch.Tensor):
+        raise TypeError("min_score must be a Python number (reading a tensor would synchronise)")
+    tau = float(min_score)
+    if not math.isfinite(tau):
+        raise ValueError("min_score must be finite")
+    batched = score.dim() == 3
+    s = score if batched else score.unsqueeze(0)
+    B, T, D = s.shape
+    if T > LSAP_MAX_SIZE or D > LSAP_MAX_SIZE or B > LSAP_MAX_BATCH:
+        raise ValueError(f"linear_assignment supports T, D <= {LSAP_MAX_SIZE} and B <= {LSAP_MAX_BATCH}; got {(B, T, D)}")
+    mask = None
+    if pair_mask is not None:
+        if pair_mask.dtype != torch.bool or pair_mask.shape != score.shape:
+            raise ValueError("pair_mask must be a bool tensor of the score's shape")
+        if pair_mask.device != score.device:
+            raise ValueError("pair_mask must be on the score's device")
+        mask = (pair_mask if batched else pair_mask.unsqueeze(0)).contiguous()
+    s = s.contiguous()
+    det_for_track = torch.empty((B, T), device=s.device, dtype=torch.int32)
+    track_for_det = torch.empty((B, D), device=s.device, dtype=torch.int32)
+    work = torch.empty((B * _lib.lib().pcreid_lsap_workspace_bytes(T, D),), device=s.device, dtype=torch.uint8)
+    _OPS.lsap(B, T, D, s, mask, tau, det_for_track, track_for_det, work)
+    det_for_track, track_for_det = det_for_track.long(), track_for_det.long()
+    if not batched:
+        return det_for_track[0], track_for_det[0]
+    return det_for_track, track_for_det
 
 
 def bf16_kmajor_image(w):

@@ -8,9 +8,14 @@
   score every admissible track x detection pair, return the dense (T, D) cost matrix (zeros where not compared).
   ``from_sweep`` runs the whole of ``__call__`` (L74-116): crop / centre / resample the sweep with the fused front-end
   (models/frontend.py replaces pc_utils.py:31-96), then encode, gate and score.
+  ``step`` is one tracker frame after that on the device: associate with ``kernels.linear_assignment`` (maximum-weight
+  matching of the class-gated pairs whose logit exceeds ``min_score``), then update the bank as the reference's
+  virtual_tracker.py:800-812 does -- matched detections through ``replace_old``, unmatched ones through ``store_new``.
+  Track lifecycle (ids, ages, deletion, motion) stays with the caller.
 """
 import torch
 
+from .. import kernels as K
 from .frontend import crop_center_resample
 
 
@@ -85,6 +90,29 @@ class PointReidentifier:
             return None, xyz_d, h_d, det_lengths
         cost, xyz_d, h_d = self(det_points, det_labels, det_lengths, track_index, track_labels)
         return cost, xyz_d, h_d, det_lengths
+
+    @torch.no_grad()
+    def step(self, sweep, bboxes, det_labels, track_index, track_labels, min_score, sample_rank=None):
+        """One frame: from_sweep, association, bank update.  Track t (a position into ``track_index``) and detection d may be
+        matched when the class gate allows it and cost[t, d] > min_score; the matching maximises the sum of
+        cost - min_score.  Matched detections replace their track's bank row in one ``replace_old`` call (the bank's policy:
+        the observation with more points is kept unless ``replace_all``); unmatched ones are appended with ``store_new``.
+        -> (track_for_det (D,) int64 position into track_index or -1, new_rows (U,) int64 bank rows created for the
+        unmatched detections in ascending detection order, cost (T, D) or None when there are no active tracks)."""
+        cost, xyz_d, h_d, len_d = self.from_sweep(sweep, bboxes, det_labels, track_index, track_labels, sample_rank)
+        dev = xyz_d.device
+        if cost is None:
+            track_for_det = torch.full((xyz_d.shape[0],), -1, dtype=torch.long, device=dev)
+        else:
+            # the gate matters: cost is 0 where a pair was not compared, and 0 can exceed a negative min_score
+            gate = class_gate(det_labels, track_labels, len_d, self.feature_set.lengths[track_index], self.use_lengths)
+            _, track_for_det = K.linear_assignment(cost, min_score, gate)
+            matched = torch.nonzero(track_for_det >= 0).squeeze(1)
+            self.feature_set.replace_old(track_index[track_for_det[matched]], xyz_d[matched], h_d[matched], len_d[matched])
+        unmatched = torch.nonzero(track_for_det < 0).squeeze(1)
+        first = len(self.feature_set)
+        self.feature_set.store_new(xyz_d[unmatched], h_d[unmatched], len_d[unmatched])
+        return track_for_det, torch.arange(first, first + unmatched.numel(), dtype=torch.long, device=dev), cost
 
     @torch.no_grad()
     def encode(self, det_points):

@@ -92,6 +92,22 @@ int pcreid_crop_tiles(int P);
 int pcreid_crop_mask(int P, int B, const float* pts, int pts_stride, const float* boxes, void* mask, int* counts, void* stream);
 int pcreid_crop_gather(int P, int B, int N, const float* pts, int pts_stride, const float* boxes, const void* mask,
                        const int* prefix, const long long* rank, float* out, void* stream);
+/* The same front-end over S sweeps in one launch per pass.  pts (sum P_s, >=3) = the sweeps one after another, row stride
+ * pts_stride; boxes (sum B_s, 7) = each scene's boxes one after another; a box is tested against its own sweep only.
+ * offsets: int32 device array [4][S + 1] of exclusive prefix sums over the scenes of
+ *   [0] P_s (points), [1] B_s (boxes), [2] ntiles_s = pcreid_crop_tiles(P_s), [3] B_s * ntiles_s (count words);
+ * total_tiles = offsets[2][S], max_boxes = max B_s, total_boxes = offsets[1][S], all known on the host.
+ * Tiles never straddle two sweeps.  Scene s's block of mask (words 32 * offsets[3][s] ..) and counts (offsets[3][s] ..) is laid out
+ * as pcreid_crop_mask lays out that sweep alone: box i of scene s (global box g = offsets[1][s] + i) at count word
+ * offsets[3][s] + i * ntiles_s.  prefix: per box, the (ntiles_s + 1) exclusive scan of its counts, box g's at
+ * offsets[3][s] + i * ntiles_s + g.  rank (sum B_s, N), out (sum B_s, N, 3) as pcreid_crop_gather.  Each box's mask words,
+ * counts and output equal pcreid_crop_mask / pcreid_crop_gather's on its own sweep (zeros for a box of an empty sweep).
+ * max_boxes > 65535 * 32 or total_boxes > 65535: PCREID_ERR_UNSUPPORTED. */
+int pcreid_crop_mask_scenes(int S, int total_tiles, int max_boxes, const float* pts, int pts_stride, const float* boxes,
+                            const int* offsets, void* mask, int* counts, void* stream);
+int pcreid_crop_gather_scenes(int S, int total_boxes, int N, const float* pts, int pts_stride, const float* boxes,
+                              const int* offsets, const void* mask, const int* prefix, const long long* rank, float* out,
+                              void* stream);
 
 /* replaces three_nn_kernel_launcher(b,n,m,unknown,known,dist2,idx,stream) (ops/interpolate/src/three_nn_cuda.cu:68-90):
  * the three nearest known (B,M,3) points of every unknown (B,N,3) point, ascending (d2, index); dist2 (B,N,3) SQUARED
@@ -263,6 +279,15 @@ int pcreid_pair_concat_head(int T, int D, int E, int G, const float* A, const fl
 int pcreid_lsap_workspace_bytes(int T, int D);   /* per problem; -1 outside the supported shapes */
 int pcreid_lsap(int B, int T, int D, const float* score, const unsigned char* mask, float min_score, int* det_for_track,
                 int* track_for_det, void* work, void* stream);
+/* B problems of different shapes (T_b, D_b) in one launch, one CTA each, the solver and the admissibility rule of pcreid_lsap.
+ * offsets: int64 device array [4][B + 1] of exclusive prefix sums over the problems of
+ *   [0] T_b, [1] D_b, [2] T_b * D_b (score / mask elements), [3] pcreid_lsap_workspace_bytes(T_b, D_b);
+ * problem b reads the row-major T_b x D_b block of score (and mask, u8 or NULL) at offsets[2][b], writes det_for_track at
+ * offsets[0][b] and track_for_det at offsets[1][b] (int32, -1 = unmatched) and uses work at byte offsets[3][b].  max_T / max_D
+ * bound every T_b / D_b (they size the CTA and its shared memory).  Each problem's result equals pcreid_lsap's on that problem
+ * alone.  0 <= max_T, max_D <= 4096 and B <= 65535, else PCREID_ERR_UNSUPPORTED; a non-finite min_score is PCREID_ERR_ARG. */
+int pcreid_lsap_blocks(int B, int max_T, int max_D, const long long* offsets, const float* score, const unsigned char* mask,
+                       float min_score, int* det_for_track, int* track_for_det, void* work, void* stream);
 
 /* ------------------------------------------------------------------ B'. fused tensor-core match path --- */
 /* Tensor-core modes of the xcorr_eff head (csrc/pair_tc.cu, csrc/pair_tc2.cu): tcgen05 kind::f16 GEMMs with fp32

@@ -60,6 +60,8 @@ _SIGS = {
     "pcreid_crop_tiles": [c_int],
     "pcreid_crop_mask": [c_int, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp],
     "pcreid_crop_gather": [c_int, c_int, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp],
+    "pcreid_crop_mask_scenes": [c_int, c_int, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp],
+    "pcreid_crop_gather_scenes": [c_int, c_int, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp],
     "pcreid_three_nn": [c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp],
     "pcreid_three_interpolate": [c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp],
     "pcreid_cn_linear": [ctypes.POINTER(LinearArgs), c_vp],
@@ -99,6 +101,7 @@ _SIGS = {
     "pcreid_pair_concat_head": [c_int, c_int, c_int, c_int] + [c_vp] * 10 + [c_float, c_vp, c_vp, c_vp],
     "pcreid_lsap_workspace_bytes": [c_int, c_int],
     "pcreid_lsap": [c_int, c_int, c_int, c_vp, c_vp, c_float, c_vp, c_vp, c_vp, c_vp],
+    "pcreid_lsap_blocks": [c_int, c_int, c_int, c_vp, c_vp, c_vp, c_float, c_vp, c_vp, c_vp, c_vp],
 }
 
 ERRORS = {1: "PCREID_ERR_ARG (bad pointer/size)", 2: "PCREID_ERR_LAUNCH (CUDA launch failed)",

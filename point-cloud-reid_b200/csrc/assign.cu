@@ -15,6 +15,8 @@
 // touched by no other thread during a Dijkstra), then the CTA selects the next column by the lexicographic minimum of
 //   (reduced distance, unassigned before assigned, column index; dummies index D + t)
 // -- a total order, so the result does not depend on the thread count or on other problems in the launch.
+// lsap_solve is that solver for one problem; lsap_kernel runs it over a batch of one shape (pcreid_lsap), lsap_blocks_kernel
+// over problems of different shapes packed one after another (pcreid_lsap_blocks).
 // Row state (u, the column of each row, the columns selected in the current Dijkstra) lives in the per-problem workspace.
 #include "../../include/pcreid.h"
 #include "common.cuh"
@@ -52,13 +54,13 @@ __host__ __device__ inline size_t lsap_work_bytes(int T, int D) {
   return (((size_t)T + steps) * 12 + 15) / 16 * 16;
 }
 
-__global__ void __launch_bounds__(MAX_THREADS) lsap_kernel(int T, int D, const float* __restrict__ score,
-                                                            const unsigned char* __restrict__ mask, float tau,
-                                                            int* __restrict__ det_for_track, int* __restrict__ track_for_det,
-                                                            unsigned char* __restrict__ work) {
-  extern __shared__ __align__(16) unsigned char smem[];
+// Solves problem (T, D) of S (row-major T x D), M (same layout or NULL) into det_for_track (T) / track_for_det (D), with the
+// workspace wb (lsap_work_bytes(T, D)) and the column state in smem (sized for at least D columns).  Called by every thread
+// of the CTA; blockDim.x is a multiple of 32 and at most MAX_THREADS.
+__device__ void lsap_solve(int T, int D, const float* __restrict__ S, const unsigned char* __restrict__ M, float tau,
+                           int* __restrict__ det_for_track, int* __restrict__ track_for_det, unsigned char* __restrict__ wb,
+                           unsigned char* smem) {
   const int nthr = blockDim.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = nthr >> 5;
-  const size_t b = blockIdx.x;
   Cand* red = reinterpret_cast<Cand*>(smem);                    // [2][32] per-warp candidates, double-buffered
   double* spc = reinterpret_cast<double*>(red + 64);            // [D] shortest reduced distance in this Dijkstra
   double* v = spc + D;                                          // [D] column duals
@@ -67,14 +69,10 @@ __global__ void __launch_bounds__(MAX_THREADS) lsap_kernel(int T, int D, const f
   unsigned char* done = reinterpret_cast<unsigned char*>(row4col + D);   // [D] column selected in this Dijkstra
 
   const int steps = (T < D ? T : D) + 1;
-  unsigned char* wb = work + b * lsap_work_bytes(T, D);
   double* u = reinterpret_cast<double*>(wb);
   double* sel_d = u + T;
   int* col4row = reinterpret_cast<int*>(sel_d + steps);         // real column, D + t for the dummy, -1 before row t is done
   int* sel_col = col4row + T;
-
-  const float* S = score + b * (size_t)T * D;
-  const unsigned char* M = mask ? mask + b * (size_t)T * D : nullptr;
   const double dtau = (double)tau;
 
   for (int j = tid; j < D; j += nthr) { v[j] = 0.0; row4col[j] = -1; }
@@ -144,9 +142,43 @@ __global__ void __launch_bounds__(MAX_THREADS) lsap_kernel(int T, int D, const f
     __syncthreads();
   }
 
-  for (int t = tid; t < T; t += nthr) det_for_track[b * T + t] = col4row[t] < D ? col4row[t] : -1;
-  for (int j = tid; j < D; j += nthr) track_for_det[b * D + j] = row4col[j];
+  for (int t = tid; t < T; t += nthr) det_for_track[t] = col4row[t] < D ? col4row[t] : -1;
+  for (int j = tid; j < D; j += nthr) track_for_det[j] = row4col[j];
 }
+
+// B problems of one shape, packed densely: problem b at b * T * D (score, mask), b * T / b * D (outputs), b * lsap_work_bytes
+__global__ void __launch_bounds__(MAX_THREADS) lsap_kernel(int T, int D, const float* __restrict__ score,
+                                                            const unsigned char* __restrict__ mask, float tau,
+                                                            int* __restrict__ det_for_track, int* __restrict__ track_for_det,
+                                                            unsigned char* __restrict__ work) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  const size_t b = blockIdx.x;
+  lsap_solve(T, D, score + b * (size_t)T * D, mask ? mask + b * (size_t)T * D : nullptr, tau, det_for_track + b * T,
+             track_for_det + b * D, work + b * lsap_work_bytes(T, D), smem);
+}
+
+// B problems of different shapes (pcreid_lsap_blocks): off = [rows | cols | score elements | workspace bytes], each (B + 1)
+// exclusive prefix sums; problem b is (off[1][b+1] - off[1][b]) x ... at those offsets
+__global__ void __launch_bounds__(MAX_THREADS) lsap_blocks_kernel(int B, const long long* __restrict__ off,
+                                                                   const float* __restrict__ score,
+                                                                   const unsigned char* __restrict__ mask, float tau,
+                                                                   int* __restrict__ det_for_track,
+                                                                   int* __restrict__ track_for_det,
+                                                                   unsigned char* __restrict__ work) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  const int b = blockIdx.x;
+  const long long* rows = off;
+  const long long* cols = off + (B + 1);
+  const long long* elems = off + 2 * (B + 1);
+  const long long* wbytes = off + 3 * (B + 1);
+  const int T = (int)(rows[b + 1] - rows[b]), D = (int)(cols[b + 1] - cols[b]);
+  lsap_solve(T, D, score + elems[b], mask ? mask + elems[b] : nullptr, tau, det_for_track + rows[b], track_for_det + cols[b],
+             work + wbytes[b], smem);
+}
+
+// threads per CTA for problems of up to D columns, and the column state they keep in shared memory
+inline int lsap_threads(int D) { return D >= MAX_THREADS ? MAX_THREADS : (D > 32 ? (D + 31) / 32 * 32 : 32); }
+inline size_t lsap_smem_bytes(int D) { return 64 * sizeof(Cand) + (size_t)D * (2 * sizeof(double) + 2 * sizeof(int) + 1); }
 
 }  // namespace
 
@@ -163,11 +195,25 @@ int pcreid_lsap(int B, int T, int D, const float* score, const unsigned char* ma
   if (B > 65535 || T > LSAP_MAX || D > LSAP_MAX) return PCREID_ERR_UNSUPPORTED;
   if (B == 0 || (T == 0 && D == 0)) return PCREID_OK;
   if ((T > 0 && D > 0 && !score) || (T > 0 && (!det_for_track || !work)) || (D > 0 && !track_for_det)) return PCREID_ERR_ARG;
-  const int nthr = D >= MAX_THREADS ? MAX_THREADS : (D > 32 ? (D + 31) / 32 * 32 : 32);
-  const size_t smem = 64 * sizeof(Cand) + (size_t)D * (2 * sizeof(double) + 2 * sizeof(int) + 1);
+  const size_t smem = lsap_smem_bytes(D);
   if (smem > 48 * 1024) cudaFuncSetAttribute(lsap_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  lsap_kernel<<<B, nthr, smem, (cudaStream_t)stream>>>(T, D, score, mask, min_score, det_for_track, track_for_det,
-                                                       (unsigned char*)work);
+  lsap_kernel<<<B, lsap_threads(D), smem, (cudaStream_t)stream>>>(T, D, score, mask, min_score, det_for_track, track_for_det,
+                                                                   (unsigned char*)work);
+  return pcreid_launch_status();
+}
+
+int pcreid_lsap_blocks(int B, int max_T, int max_D, const long long* offsets, const float* score, const unsigned char* mask,
+                       float min_score, int* det_for_track, int* track_for_det, void* work, void* stream) {
+  if (B < 0 || max_T < 0 || max_D < 0 || !std::isfinite(min_score)) return PCREID_ERR_ARG;
+  if (B > 65535 || max_T > LSAP_MAX || max_D > LSAP_MAX) return PCREID_ERR_UNSUPPORTED;
+  if (B == 0 || (max_T == 0 && max_D == 0)) return PCREID_OK;
+  if (!offsets || (max_T > 0 && max_D > 0 && !score) || (max_T > 0 && (!det_for_track || !work)) ||
+      (max_D > 0 && !track_for_det))
+    return PCREID_ERR_ARG;
+  const size_t smem = lsap_smem_bytes(max_D);
+  if (smem > 48 * 1024) cudaFuncSetAttribute(lsap_blocks_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  lsap_blocks_kernel<<<B, lsap_threads(max_D), smem, (cudaStream_t)stream>>>(B, offsets, score, mask, min_score, det_for_track,
+                                                                              track_for_det, (unsigned char*)work);
   return pcreid_launch_status();
 }
 

@@ -56,15 +56,14 @@ __device__ __forceinline__ bool in_box(const BoxC& k, float px, float py, float 
   return ((double)lx > -k.hl) & ((double)lx < k.hl) & ((double)ly > -k.hw) & ((double)ly < k.hw);
 }
 
-// pass 1: mask[b][tile][32] (bit i of word w <-> point tile*1024 + 32 w + i), counts[b][tile]
-__global__ void __launch_bounds__(256) crop_mask_kernel(int P, int B, int ntiles, const float* __restrict__ pts, int ps,
-                                                        const float* __restrict__ boxes, uint32_t* __restrict__ mask,
-                                                        int* __restrict__ counts) {
+// pass 1 for one tile of one sweep and up to BB boxes b0 .. b0 + nb - 1 of that sweep:
+//   mask[b][tile][32] (bit i of word w <-> point tile*1024 + 32 w + i), counts[b][tile]
+__device__ __forceinline__ void crop_mask_tile(int P, int nb, int ntiles, int tile, const float* __restrict__ pts, int ps,
+                                               const float* __restrict__ boxes, uint32_t* __restrict__ mask,
+                                               int* __restrict__ counts) {
   __shared__ BoxC bc[BB];
   __shared__ int cnt[BB];
-  const int tile = blockIdx.x, b0 = blockIdx.y * BB;
-  const int nb = min(BB, B - b0);
-  if (threadIdx.x < nb) { bc[threadIdx.x] = box_consts(boxes + (size_t)(b0 + threadIdx.x) * 7); cnt[threadIdx.x] = 0; }
+  if (threadIdx.x < nb) { bc[threadIdx.x] = box_consts(boxes + (size_t)threadIdx.x * 7); cnt[threadIdx.x] = 0; }
   float px[4], py[4], pz[4];
   bool live[4];
 #pragma unroll
@@ -83,37 +82,66 @@ __global__ void __launch_bounds__(256) crop_mask_kernel(int P, int B, int ntiles
     for (int j = 0; j < 4; ++j) {
       const uint32_t w = __ballot_sync(FULL_MASK, live[j] && in_box(k, px[j], py[j], pz[j]));
       if (lane == 0) {
-        mask[((size_t)(b0 + i) * ntiles + tile) * 32 + j * 8 + warp] = w;
+        mask[((size_t)i * ntiles + tile) * 32 + j * 8 + warp] = w;
         c += __popc(w);
       }
     }
     if (lane == 0 && c) atomicAdd(&cnt[i], c);
   }
   __syncthreads();
-  if (threadIdx.x < nb) counts[(size_t)(b0 + threadIdx.x) * ntiles + tile] = cnt[threadIdx.x];
+  if (threadIdx.x < nb) counts[(size_t)threadIdx.x * ntiles + tile] = cnt[threadIdx.x];
 }
 
-// pass 2: out[b][n] = Rz(yaw)-frame coordinates of the sample_rank[b][n]-th in-box point (zeros for an empty box)
-//   prefix[b][0..ntiles] exclusive scan of counts
-__global__ void __launch_bounds__(128) crop_gather_kernel(int P, int N, int ntiles, const float* __restrict__ pts, int ps,
-                                                          const float* __restrict__ boxes, const uint32_t* __restrict__ mask,
-                                                          const int* __restrict__ prefix, const long long* __restrict__ rank,
-                                                          float* __restrict__ out) {
-  const int b = blockIdx.y, n = blockIdx.x * blockDim.x + threadIdx.x;
-  if (n >= N) return;
-  float* o = out + ((size_t)b * N + n) * 3;
-  const int* pf = prefix + (size_t)b * (ntiles + 1);
-  const int len = pf[ntiles];
-  if (len <= 0) { o[0] = 0.f; o[1] = 0.f; o[2] = 0.f; return; }
-  long long r = rank[(size_t)b * N + n];
-  r = r < 0 ? 0 : (r >= len ? len - 1 : r);
-  int lo = 0, hi = ntiles;                       // largest tile with prefix[tile] <= r
+__global__ void __launch_bounds__(256) crop_mask_kernel(int P, int B, int ntiles, const float* __restrict__ pts, int ps,
+                                                        const float* __restrict__ boxes, uint32_t* __restrict__ mask,
+                                                        int* __restrict__ counts) {
+  const int b0 = blockIdx.y * BB;
+  crop_mask_tile(P, min(BB, B - b0), ntiles, blockIdx.x, pts, ps, boxes + (size_t)b0 * 7, mask + (size_t)b0 * ntiles * 32,
+                 counts + (size_t)b0 * ntiles);
+}
+
+// segment of a prefix array holding x: the largest s with off[s] <= x (off nondecreasing, off[0] <= x < off[S])
+__device__ __forceinline__ int segment_of(const int* __restrict__ off, int S, int x) {
+  int lo = 0, hi = S;
   while (hi - lo > 1) {
     const int mid = (lo + hi) >> 1;
-    if (pf[mid] <= r) lo = mid; else hi = mid;
+    if (off[mid] <= x) lo = mid; else hi = mid;
   }
+  return lo;
+}
+
+// offsets of the segmented front-end (pcreid_crop_mask_scenes): off = [points | boxes | tiles | count words], each (S + 1)
+struct SceneOff {
+  const int *pt, *box, *tile, *cnt;
+  __device__ SceneOff(const int* off, int S) : pt(off), box(off + (S + 1)), tile(off + 2 * (S + 1)), cnt(off + 3 * (S + 1)) {}
+};
+
+// one CTA per (tile of scene s, box group y of scene s): scene s's block of mask / counts is laid out as pcreid_crop_mask's for
+// that sweep alone
+__global__ void __launch_bounds__(256) crop_mask_scenes_kernel(int S, const float* __restrict__ pts, int ps,
+                                                               const float* __restrict__ boxes, const int* __restrict__ off,
+                                                               uint32_t* __restrict__ mask, int* __restrict__ counts) {
+  const SceneOff o(off, S);
+  const int s = segment_of(o.tile, S, blockIdx.x);
+  const int B = o.box[s + 1] - o.box[s], b0 = blockIdx.y * BB;
+  if (b0 >= B) return;
+  const int ntiles = o.tile[s + 1] - o.tile[s];
+  const size_t c0 = (size_t)o.cnt[s] + (size_t)b0 * ntiles;
+  crop_mask_tile(o.pt[s + 1] - o.pt[s], min(BB, B - b0), ntiles, blockIdx.x - o.tile[s], pts + (size_t)o.pt[s] * ps, ps,
+                 boxes + (size_t)(o.box[s] + b0) * 7, mask + c0 * 32, counts + c0);
+}
+
+// pass 2 for one output slot: o = Rz(yaw)-frame coordinates of the r-th in-box point of the box (zeros for an empty box)
+//   pf[0..ntiles]: exclusive scan of the box's counts, mw: the box's mask words
+__device__ __forceinline__ void crop_gather_one(int ntiles, const float* __restrict__ pts, int ps, const float* __restrict__ bx,
+                                                const uint32_t* __restrict__ mw, const int* __restrict__ pf, long long r,
+                                                float* __restrict__ o) {
+  const int len = pf[ntiles];
+  if (len <= 0) { o[0] = 0.f; o[1] = 0.f; o[2] = 0.f; return; }
+  r = r < 0 ? 0 : (r >= len ? len - 1 : r);
+  const int lo = segment_of(pf, ntiles, (int)r);  // largest tile with prefix[tile] <= r
   int rem = (int)r - pf[lo];
-  const uint32_t* mw = mask + ((size_t)b * ntiles + lo) * 32;
+  mw += (size_t)lo * 32;
   int word = 0;
   uint32_t w = mw[0];
   while (rem >= __popc(w)) { rem -= __popc(w); w = mw[++word]; }     // mask words are stored as [pass j][warp]: word = 8 j + warp
@@ -121,13 +149,39 @@ __global__ void __launch_bounds__(128) crop_gather_kernel(int P, int N, int ntil
   const int bit = __ffs(w) - 1;
   const int p = lo * CT + (word >> 3) * 256 + (word & 7) * 32 + bit;
   const float* q = pts + (size_t)p * ps;
-  const float* bx = boxes + (size_t)b * 7;
   float s, c;
   sincosf(bx[6], &s, &c);
   const float dx = q[0] - bx[0], dy = q[1] - bx[1];
   o[0] = c * dx - s * dy;                        // inverse of [Rz(-yaw) | centre] applied to the point (pc_utils.py:62-76)
   o[1] = s * dx + c * dy;
   o[2] = q[2] - bx[2];
+}
+
+// out[b][n] for rank[b][n]; prefix[b][0..ntiles] exclusive scan of counts
+__global__ void __launch_bounds__(128) crop_gather_kernel(int P, int N, int ntiles, const float* __restrict__ pts, int ps,
+                                                          const float* __restrict__ boxes, const uint32_t* __restrict__ mask,
+                                                          const int* __restrict__ prefix, const long long* __restrict__ rank,
+                                                          float* __restrict__ out) {
+  const int b = blockIdx.y, n = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= N) return;
+  crop_gather_one(ntiles, pts, ps, boxes + (size_t)b * 7, mask + (size_t)b * ntiles * 32, prefix + (size_t)b * (ntiles + 1),
+                  rank[(size_t)b * N + n], out + ((size_t)b * N + n) * 3);
+}
+
+// global box g of scene s (local index i): mask / counts at cnt[s] + i * ntiles_s, prefix at cnt[s] + i * ntiles_s + g
+__global__ void __launch_bounds__(128) crop_gather_scenes_kernel(int S, int N, const float* __restrict__ pts, int ps,
+                                                                 const float* __restrict__ boxes, const int* __restrict__ off,
+                                                                 const uint32_t* __restrict__ mask,
+                                                                 const int* __restrict__ prefix,
+                                                                 const long long* __restrict__ rank, float* __restrict__ out) {
+  const int g = blockIdx.y, n = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= N) return;
+  const SceneOff o(off, S);
+  const int s = segment_of(o.box, S, g);
+  const int ntiles = o.tile[s + 1] - o.tile[s];
+  const size_t c0 = (size_t)o.cnt[s] + (size_t)(g - o.box[s]) * ntiles;
+  crop_gather_one(ntiles, pts + (size_t)o.pt[s] * ps, ps, boxes + (size_t)g * 7, mask + c0 * 32, prefix + c0 + g,
+                  rank[(size_t)g * N + n], out + ((size_t)g * N + n) * 3);
 }
 
 }  // namespace
@@ -154,6 +208,29 @@ int pcreid_crop_gather(int P, int B, int N, const float* pts, int pts_stride, co
   const int ntiles = (P + CT - 1) / CT;
   crop_gather_kernel<<<dim3((N + 127) / 128, B), 128, 0, (cudaStream_t)stream>>>(P, N, ntiles, pts, pts_stride, boxes,
                                                                                  (const uint32_t*)mask, prefix, rank, out);
+  return pcreid_launch_status();
+}
+
+int pcreid_crop_mask_scenes(int S, int total_tiles, int max_boxes, const float* pts, int pts_stride, const float* boxes,
+                            const int* offsets, void* mask, int* counts, void* stream) {
+  if (S < 0 || total_tiles < 0 || max_boxes < 0) return PCREID_ERR_ARG;
+  if (S == 0 || total_tiles == 0 || max_boxes == 0) return PCREID_OK;
+  if (!pts || !boxes || !offsets || !mask || !counts || pts_stride < 3) return PCREID_ERR_ARG;
+  if ((max_boxes + BB - 1) / BB > 65535) return PCREID_ERR_UNSUPPORTED;
+  crop_mask_scenes_kernel<<<dim3(total_tiles, (max_boxes + BB - 1) / BB), 256, 0, (cudaStream_t)stream>>>(
+      S, pts, pts_stride, boxes, offsets, (uint32_t*)mask, counts);
+  return pcreid_launch_status();
+}
+
+int pcreid_crop_gather_scenes(int S, int total_boxes, int N, const float* pts, int pts_stride, const float* boxes,
+                              const int* offsets, const void* mask, const int* prefix, const long long* rank, float* out,
+                              void* stream) {
+  if (S < 0 || total_boxes < 0 || N < 0) return PCREID_ERR_ARG;
+  if (S == 0 || total_boxes == 0 || N == 0) return PCREID_OK;
+  if (!boxes || !offsets || !prefix || !rank || !out || pts_stride < 3) return PCREID_ERR_ARG;
+  if (total_boxes > 65535) return PCREID_ERR_UNSUPPORTED;
+  crop_gather_scenes_kernel<<<dim3((N + 127) / 128, total_boxes), 128, 0, (cudaStream_t)stream>>>(
+      S, N, pts, pts_stride, boxes, offsets, (const uint32_t*)mask, prefix, rank, out);
   return pcreid_launch_status();
 }
 

@@ -580,6 +580,47 @@ def linear_assignment(score, min_score, pair_mask=None):
     return det_for_track, track_for_det
 
 
+def linear_assignment_blocks(score, shapes, min_score, pair_mask=None):
+    """linear_assignment over B problems of different shapes in one launch (pcreid_lsap_blocks), e.g. one per scene.
+    score: 1-D CUDA float32 of sum T_b * D_b, problem b's row-major (T_b, D_b) block after problem b-1's; shapes: host sequence
+    of (T_b, D_b); pair_mask: bool, packed like score, or None.  Each problem's result equals linear_assignment on its block.
+    -> packed int64 (det_for_track (sum T_b,), track_for_det (sum D_b,)) on the device, -1 = unmatched.  Validates the shapes on
+    the host and never reads device memory back (no host synchronisation)."""
+    _need_cuda(score, pair_mask)
+    if score.dtype != torch.float32 or score.dim() != 1:
+        raise TypeError("score must be 1-D float32 (problems packed one after another)")
+    if isinstance(min_score, torch.Tensor):
+        raise TypeError("min_score must be a Python number (reading a tensor would synchronise)")
+    tau = float(min_score)
+    if not math.isfinite(tau):
+        raise ValueError("min_score must be finite")
+    shapes = [(int(t), int(d)) for t, d in shapes]
+    B = len(shapes)
+    if B > LSAP_MAX_BATCH or any(t < 0 or d < 0 or t > LSAP_MAX_SIZE or d > LSAP_MAX_SIZE for t, d in shapes):
+        raise ValueError(f"linear_assignment_blocks supports 0 <= T, D <= {LSAP_MAX_SIZE} and at most {LSAP_MAX_BATCH} problems")
+    L = _lib.lib()
+    offs = [[0] for _ in range(4)]
+    for t, d in shapes:
+        for row, v in zip(offs, (t, d, t * d, L.pcreid_lsap_workspace_bytes(t, d))):
+            row.append(row[-1] + v)
+    if score.numel() != offs[2][-1]:
+        raise ValueError(f"score holds {score.numel()} elements; the shapes need {offs[2][-1]}")
+    if pair_mask is not None:
+        if pair_mask.dtype != torch.bool or pair_mask.shape != score.shape:
+            raise ValueError("pair_mask must be a bool tensor of the score's shape")
+        if pair_mask.device != score.device:
+            raise ValueError("pair_mask must be on the score's device")
+        pair_mask = pair_mask.contiguous()
+    dev = score.device
+    det_for_track = torch.empty((offs[0][-1],), device=dev, dtype=torch.int32)
+    track_for_det = torch.empty((offs[1][-1],), device=dev, dtype=torch.int32)
+    work = torch.empty((offs[3][-1],), device=dev, dtype=torch.uint8)
+    off = torch.tensor(offs, dtype=torch.int64).pin_memory().to(dev, non_blocking=True)
+    _OPS.lsap_blocks(B, max((t for t, _ in shapes), default=0), max((d for _, d in shapes), default=0), off, score.contiguous(),
+                     pair_mask, tau, det_for_track, track_for_det, work)
+    return det_for_track.long(), track_for_det.long()
+
+
 def bf16_kmajor_image(w):
     """torch weight (N, K) -> bf16 K-major tcgen05 operand image [K/8][N][8] (uint8 view)."""
     n, kd = w.shape

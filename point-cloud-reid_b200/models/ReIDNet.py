@@ -419,50 +419,73 @@ class ReIDNet(nn.Module):
 
     def _match_all_pairs(self, h_t, xyz_t, h_d, xyz_d, pair_mask=None, chunk=8192, _exact_chunk=False):
         with torch.no_grad():
-            h_t, h_d = _cn(h_t), _cn(h_d)
-            xyz_t, xyz_d = xyz_t.float().contiguous(), xyz_d.float().contiguous()
-            T, D = h_t.shape[0], h_d.shape[0]
-            dev = h_t.device
             if self.match_type == 'concat':
-                return self._concat_all_pairs(h_t, h_d, pair_mask)
-            out = torch.zeros((T, D), device=dev, dtype=torch.float32)
-            fused = None
-            if self.match_mode in self.TC_MODES:
-                from . import fused_pairs
-                if fused_pairs.supported(self, h_t.shape[2]) and h_t.shape[2] == h_d.shape[2]:
-                    fused = self.fused_matcher()
-                    pk_t, pk_d = fused.prepare(h_t, xyz_t), fused.prepare(h_d, xyz_d)
-                    if not _exact_chunk:
-                        chunk = max(chunk, 65536 * 256 // h_t.shape[2])
-            if pair_mask is None:
-                pairs = None
-                total = T * D
-            else:
-                pairs = pair_mask.nonzero()
-                total = pairs.shape[0]
+                return self._concat_all_pairs(_cn(h_t), _cn(h_d), pair_mask)
+            ctx, chunk = self._pair_context(h_t, xyz_t, h_d, xyz_d, chunk, _exact_chunk)
+            T, D = ctx[0].shape[0], ctx[2].shape[0]
+            fused = ctx[4]
+            out = torch.zeros((T, D), device=ctx[0].device, dtype=torch.float32)
             flat = out.view(-1)
-            with self._tc_match(fused is not None):
-                if pairs is None and fused is not None and D > 0:
+            if pair_mask is None and fused is not None and D > 0:
+                with self._tc_match(True):
                     rows_per_chunk = max(1, chunk // D)                          # dense all-pairs: whole rows per chunk
                     for r0 in range(0, T, rows_per_chunk):
                         nrows = min(rows_per_chunk, T - r0)
-                        flat[r0 * D:(r0 + nrows) * D] = fused.match(pk_t, pk_d, None, None, dense=(r0, nrows, D))
-                    return out
-                for s in range(0, total, chunk):
-                    e = min(total, s + chunk)
-                    if pairs is None:
-                        lin = torch.arange(s, e, device=dev)
-                        ti, dj = lin // D, lin % D
-                    else:
-                        ti, dj = pairs[s:e, 0], pairs[s:e, 1]
-                        lin = ti * D + dj
-                    if fused is not None:
-                        flat[lin] = fused.match(pk_t, pk_d, ti, dj)
-                    elif self.match_type == 'xcorr_eff':
-                        flat[lin] = self._xcorr_pairs(h_t, xyz_t, h_d, xyz_d, _i32(ti), _i32(dj))
-                    else:
-                        flat[lin] = self._xcorr_search_pairs(h_t, xyz_t, h_d, xyz_d, _i32(ti), _i32(dj))
+                        flat[r0 * D:(r0 + nrows) * D] = fused.match(ctx[5], ctx[6], None, None, dense=(r0, nrows, D))
+                return out
+            pairs = None if pair_mask is None else pair_mask.nonzero()
+            total = T * D if pairs is None else pairs.shape[0]
+            for s in range(0, total, chunk):
+                e = min(total, s + chunk)
+                if pairs is None:
+                    lin = torch.arange(s, e, device=out.device)
+                    ti, dj = lin // D, lin % D
+                else:
+                    ti, dj = pairs[s:e, 0], pairs[s:e, 1]
+                    lin = ti * D + dj
+                flat[lin] = self._pair_logits(ctx, ti, dj)
             return out
+
+    def match_pairs(self, h_t, xyz_t, h_d, xyz_d, ti, dj, chunk=8192):
+        """logits (P,) of the listed pairs (track ti[p], detection dj[p]), any order, repeats allowed: the entries
+        match_all_pairs(..., pair_mask) gives those pairs.  One call serves the pairs of many scenes: a pair's logit depends on
+        its two objects only.  'concat' models score through match_all_pairs (the dense pooled head)."""
+        if self.match_type == 'concat':
+            raise NotImplementedError("'concat' scores whole (T, D) blocks: use match_all_pairs(..., pair_mask=...)")
+        with torch.no_grad():
+            ctx, chunk = self._pair_context(h_t, xyz_t, h_d, xyz_d, chunk, False)
+            P = ti.shape[0]
+            if dj.shape[0] != P:
+                raise ValueError("ti and dj must list the same number of pairs")
+            out = torch.empty((P,), device=ctx[0].device, dtype=torch.float32)
+            for s in range(0, P, chunk):
+                e = min(P, s + chunk)
+                out[s:e] = self._pair_logits(ctx, ti[s:e], dj[s:e])
+            return out
+
+    def _pair_context(self, h_t, xyz_t, h_d, xyz_d, chunk, _exact_chunk):
+        """per-object work of the pair scorer -> ((h_t, xyz_t, h_d, xyz_d, fused matcher or None, packed t, packed d), chunk)"""
+        h_t, h_d = _cn(h_t), _cn(h_d)
+        xyz_t, xyz_d = xyz_t.float().contiguous(), xyz_d.float().contiguous()
+        fused = pk_t = pk_d = None
+        if self.match_mode in self.TC_MODES:
+            from . import fused_pairs
+            if fused_pairs.supported(self, h_t.shape[2]) and h_t.shape[2] == h_d.shape[2]:
+                fused = self.fused_matcher()
+                pk_t, pk_d = fused.prepare(h_t, xyz_t), fused.prepare(h_d, xyz_d)
+                if not _exact_chunk:
+                    chunk = max(chunk, 65536 * 256 // h_t.shape[2])
+        return (h_t, xyz_t, h_d, xyz_d, fused, pk_t, pk_d), chunk
+
+    def _pair_logits(self, ctx, ti, dj):
+        """logits of one chunk of listed pairs: the one pair-list path of match_pairs and match_all_pairs"""
+        h_t, xyz_t, h_d, xyz_d, fused, pk_t, pk_d = ctx
+        with self._tc_match(fused is not None):
+            if fused is not None:
+                return fused.match(pk_t, pk_d, ti, dj)
+            if self.match_type == 'xcorr_eff':
+                return self._xcorr_pairs(h_t, xyz_t, h_d, xyz_d, _i32(ti), _i32(dj))
+            return self._xcorr_search_pairs(h_t, xyz_t, h_d, xyz_d, _i32(ti), _i32(dj))
 
     def pooled_embedding(self, h):
         """'concat' match type: the per-object vector the head consumes (max over the channel axis, ReIDNet.py:455-458);

@@ -53,3 +53,63 @@ def crop_center_resample(bboxes, pts, subsample_number, sample_rank=None, genera
     out = torch.empty((B, N, 3), device=pts.device, dtype=torch.float32)
     _OPS.crop_gather(P, B, N, pts, pts.shape[1], bboxes, mask, prefix, sample_rank, out)
     return out.unsqueeze(0), lengths.unsqueeze(0)
+
+
+def _to_device_async(host, dtype, device):
+    """host list -> device tensor through pinned memory: an asynchronous copy, no synchronisation with the device."""
+    t = torch.tensor(host, dtype=dtype)
+    return t.pin_memory().to(device, non_blocking=True) if torch.device(device).type == "cuda" else t.to(device)
+
+
+def crop_center_resample_scenes(bboxes, pts, box_counts, point_counts, subsample_number, sample_rank=None):
+    """crop_center_resample over S sweeps in one launch per pass (pcreid_crop_mask_scenes / pcreid_crop_gather_scenes).
+    pts (sum P_s, >=3) = the sweeps one after another, bboxes (sum B_s, 7) = each scene's boxes one after another; box_counts /
+    point_counts: host sequences of B_s / P_s.  Each box is cropped from its own sweep only.
+    -> (out (sum B_s, N, 3), lengths (sum B_s,) int64).  With ``sample_rank`` (sum B_s, N) int64 given, scene s's rows equal
+    crop_center_resample on that scene with its rows of sample_rank; without it, ranks are drawn on the device (the same
+    distribution, not the same draws)."""
+    if not (bboxes.is_cuda and pts.is_cuda):
+        raise RuntimeError("pcreid_b200 kernels need CUDA tensors (there is no CPU fallback)")
+    box_counts, point_counts = [int(b) for b in box_counts], [int(p) for p in point_counts]
+    S, N, dev = len(box_counts), int(subsample_number), pts.device
+    if len(point_counts) != S or min(box_counts + point_counts, default=0) < 0:
+        raise ValueError("box_counts and point_counts must hold one non-negative size per scene")
+    if bboxes.dtype != torch.float32 or pts.dtype != torch.float32 or bboxes.dim() != 2 or bboxes.shape[1] != 7:
+        raise ValueError("bboxes must be float32 (sum B_s, 7) and pts float32 (sum P_s, >=3)")
+    if pts.dim() != 2 or pts.shape[1] < 3:
+        raise ValueError("pts must be (sum P_s, >=3)")
+    if bboxes.shape[0] != sum(box_counts) or pts.shape[0] != sum(point_counts):
+        raise ValueError("bboxes / pts rows must be the sums of box_counts / point_counts")
+    B = bboxes.shape[0]
+    L = _lib.lib()
+    nt = [L.pcreid_crop_tiles(p) for p in point_counts]
+    offs = [[0] for _ in range(4)]
+    for p, b, t in zip(point_counts, box_counts, nt):
+        for row, v in zip(offs, (p, b, t, b * t)):
+            row.append(row[-1] + v)
+    C = offs[3][-1]
+    if C * 32 >= 1 << 31:
+        raise ValueError("mask of the segmented front-end exceeds 2^31 words: split the scenes over several calls")
+    off = _to_device_async(offs, torch.int32, dev)
+    bboxes, pts = bboxes.contiguous(), pts.contiguous()
+    mask = torch.empty((C, 32), device=dev, dtype=torch.int32)
+    counts = torch.empty((C,), device=dev, dtype=torch.int32)
+    if C > 0:                   # else no box has a tile: every crop is empty
+        _OPS.crop_mask_scenes(S, offs[2][-1], max(box_counts), pts, pts.shape[1], bboxes, off, mask, counts)
+    # per box: its ntiles count words, and its prefix (ntiles + 1) at count word + global box index
+    nt_box = _to_device_async([t for b, t in zip(box_counts, nt) for _ in range(b)], torch.int64, dev)
+    seg = torch.repeat_interleave(torch.arange(B, device=dev), nt_box, output_size=C)
+    incl = counts.cumsum(0, dtype=torch.int64)
+    start = torch.cumsum(nt_box, 0) - nt_box                                  # first count word of each box
+    within = incl - (incl - counts)[start[seg]]                             # inclusive scan inside each box
+    prefix = torch.zeros((B + C,), device=dev, dtype=torch.int32)
+    prefix[torch.arange(C, device=dev) + seg + 1] = within.to(torch.int32)
+    lengths = torch.zeros((B,), device=dev, dtype=torch.int64).index_add_(0, seg, counts.to(torch.int64))
+    if sample_rank is None:
+        sample_rank = (torch.rand((B, N), device=dev) * lengths[:, None]).long()
+    sample_rank = sample_rank.to(device=dev, dtype=torch.int64).contiguous()
+    if sample_rank.shape != (B, N):
+        raise ValueError(f"sample_rank must be ({B}, {N})")
+    out = torch.empty((B, N, 3), device=dev, dtype=torch.float32)
+    _OPS.crop_gather_scenes(S, B, N, pts, pts.shape[1], bboxes, off, mask, prefix, sample_rank, out)
+    return out, lengths

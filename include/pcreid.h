@@ -289,6 +289,42 @@ int pcreid_lsap(int B, int T, int D, const float* score, const unsigned char* ma
 int pcreid_lsap_blocks(int B, int max_T, int max_D, const long long* offsets, const float* score, const unsigned char* mask,
                        float min_score, int* det_for_track, int* track_for_det, void* work, void* stream);
 
+/* Device-resident track table (csrc/tracks.cu): S scenes x C slots, slot arrays flat over S * C (global row r = s * C + slot):
+ * alive u8, track_id i64, label i32, length i32 (points of the kept observation), age i32 (steps since the last match),
+ * hits i32, box (7 f32: the last matched detection's box); per scene next_id i64, dropped i64, active_count i32, and the
+ * active list active[s * C ..] = global rows of the alive slots in ascending slot order (active_count[s] of them).
+ * offsets: int64 device array [3][S + 1] of exclusive prefix sums over the scenes of
+ *   [0] A_s (active tracks entering the step), [1] D_s (detections), [2] A_s * D_s (gate elements);
+ * a scene without a frame passes A_s = D_s = 0 and is left unchanged.  Detection arrays are packed over the scenes at offsets[1].
+ * 1 <= C <= 4096, every D_s <= 4096 (max_D bounds them), S <= 65535, else PCREID_ERR_UNSUPPORTED; bad sizes or missing
+ * pointers are PCREID_ERR_ARG, answered before any CUDA call.
+ *
+ * pcreid_track_gate_blocks: gate (sum A_s * D_s) u8, scene s's row-major (A_s, D_s) block at offsets[2][s] (the packing of
+ *   pcreid_lsap_blocks): track t = row active[s * C + t], detection d.  1 when both labels are equal and in [0, num_classes),
+ *   both lengths >= min_points when use_lengths, and, when r2 (num_classes f32, the squared radius per class) is given,
+ *   fl(fl(dx * dx) + fl(dy * dy)) <= r2[label] with dx, dy = fl(track box - detection box) in x, y (no contraction).
+ * pcreid_track_update: one CTA per scene.  track_for_det (sum D_s) int64 = position in the scene's active list or -1 (the
+ *   output of pcreid_lsap_blocks on the gate's blocks; every position at most once).  In order:
+ *   1. matched t <- d: age 0, hits + 1, box = d's; the observation (length, rows) is replaced when replace_all or
+ *      length <= d's length.  2. unmatched active tracks: age + 1, freed when max_age >= 0 and age > max_age (-1: never).
+ *   3. the k-th unmatched detection (ascending d) takes the k-th lowest free slot with id next_id + k, age 0, hits 1 and its
+ *      label, length and box; without a free slot its id is -1 and dropped[s] + 1.  next_id advances by the number stored.
+ *   4. the active list and active_count are rebuilt.
+ *   Writes det_track_id (sum D_s) int64 and det_row (sum D_s) int32: the global row receiving d's observation, -1 if none.
+ * pcreid_track_scatter: for every d < n_det with det_row[d] >= 0, the xyz_bytes bytes of det_xyz row d to xyz row det_row[d],
+ *   and the same for the feature rows (rows are opaque bytes). */
+int pcreid_track_gate_blocks(int S, int C, int max_A, int max_D, const long long* offsets, const int* active, const int* label,
+                             const int* length, const float* box, const int* det_label, const int* det_length,
+                             const float* det_box, int num_classes, int min_points, int use_lengths, const float* r2,
+                             unsigned char* gate, void* stream);
+int pcreid_track_update(int S, int C, int max_D, const long long* offsets, const long long* track_for_det, const int* det_label,
+                        const int* det_length, const float* det_box, int max_age, int replace_all, unsigned char* alive,
+                        long long* track_id, int* label, int* length, int* age, int* hits, float* box, long long* next_id,
+                        long long* dropped, int* active, int* active_count, long long* det_track_id, int* det_row,
+                        void* stream);
+int pcreid_track_scatter(int n_det, const int* det_row, long long xyz_bytes, const void* det_xyz, void* xyz,
+                         long long feat_bytes, const void* det_feat, void* feat, void* stream);
+
 /* ------------------------------------------------------------------ B'. fused tensor-core match path --- */
 /* Tensor-core modes of the xcorr_eff head (csrc/pair_tc.cu, csrc/pair_tc2.cu): tcgen05 kind::f16 GEMMs with fp32
  * accumulation and fp32 norms.  `fmt` selects the 16-bit operand format of EVERY operand image of a call chain:

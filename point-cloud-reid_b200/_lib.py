@@ -102,6 +102,9 @@ _SIGS = {
     "pcreid_lsap_workspace_bytes": [c_int, c_int],
     "pcreid_lsap": [c_int, c_int, c_int, c_vp, c_vp, c_float, c_vp, c_vp, c_vp, c_vp],
     "pcreid_lsap_blocks": [c_int, c_int, c_int, c_vp, c_vp, c_vp, c_float, c_vp, c_vp, c_vp, c_vp],
+    "pcreid_track_gate_blocks": [c_int] * 4 + [c_vp] * 8 + [c_int] * 3 + [c_vp, c_vp, c_vp],
+    "pcreid_track_update": [c_int] * 3 + [c_vp] * 5 + [c_int, c_int] + [c_vp] * 13 + [c_vp],
+    "pcreid_track_scatter": [c_int, c_vp, c_ll, c_vp, c_vp, c_ll, c_vp, c_vp, c_vp],
 }
 
 ERRORS = {1: "PCREID_ERR_ARG (bad pointer/size)", 2: "PCREID_ERR_LAUNCH (CUDA launch failed)",

@@ -621,6 +621,120 @@ def linear_assignment_blocks(score, shapes, min_score, pair_mask=None):
     return det_for_track.long(), track_for_det.long()
 
 
+TRACK_MAX_CAPACITY, TRACK_MAX_SCENES = 4096, 65535
+# the device state of a track table (models/tracking.py, TrackTable): (attribute, dtype, trailing shape); per slot (S, C, ...),
+# per scene (S,)
+TRACK_SLOT_FIELDS = (("alive", torch.bool, ()), ("track_id", torch.int64, ()), ("label", torch.int32, ()),
+                     ("length", torch.int32, ()), ("age", torch.int32, ()), ("hits", torch.int32, ()),
+                     ("box", torch.float32, (7,)), ("active", torch.int32, ()))
+TRACK_SCENE_FIELDS = (("next_id", torch.int64), ("dropped", torch.int64), ("count", torch.int32))
+
+
+def _track_state(table):
+    """checks the table's tensors (pcreid_track_* layout) on the host -> (S, C, device)"""
+    S, C = table.alive.shape
+    if C < 1 or C > TRACK_MAX_CAPACITY or S > TRACK_MAX_SCENES:
+        raise ValueError(f"track tables support 1 <= capacity <= {TRACK_MAX_CAPACITY} and at most {TRACK_MAX_SCENES} scenes")
+    dev = table.alive.device
+    _need_cuda(table.alive)
+    for name, dtype, tail in TRACK_SLOT_FIELDS:
+        t = getattr(table, name)
+        if t.dtype != dtype or tuple(t.shape) != (S, C) + tail or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"table.{name} must be contiguous {dtype} of shape {(S, C) + tail} on {dev}")
+    for name, dtype in TRACK_SCENE_FIELDS:
+        t = getattr(table, name)
+        if t.dtype != dtype or tuple(t.shape) != (S,) or t.device != dev:
+            raise ValueError(f"table.{name} must be {dtype} of shape {(S,)} on {dev}")
+    return S, C, dev
+
+
+def _track_offsets(shapes, S, C, dev):
+    """host (A_s, D_s) per scene -> (shapes, host prefix sums [3][S + 1], the same on the device through pinned memory)"""
+    shapes = [(int(a), int(d)) for a, d in shapes]
+    if len(shapes) != S:
+        raise ValueError(f"{len(shapes)} block shapes for {S} scenes")
+    if any(a < 0 or d < 0 or a > C or d > TRACK_MAX_CAPACITY for a, d in shapes):
+        raise ValueError(f"every scene needs 0 <= A_s <= capacity ({C}) and 0 <= D_s <= {TRACK_MAX_CAPACITY}")
+    offs = [[0] for _ in range(3)]
+    for a, d in shapes:
+        for row, v in zip(offs, (a, d, a * d)):
+            row.append(row[-1] + v)
+    return shapes, offs, torch.tensor(offs, dtype=torch.int64).pin_memory().to(dev, non_blocking=True)
+
+
+def _det_arrays(n, det_label, det_length, det_box, dev):
+    for name, t, dtype, shape in (("det_label", det_label, torch.int32, (n,)), ("det_length", det_length, torch.int32, (n,)),
+                                  ("det_box", det_box, torch.float32, (n, 7))):
+        if t.dtype != dtype or tuple(t.shape) != shape or t.device != dev:
+            raise ValueError(f"{name} must be {dtype} of shape {shape} on {dev}")
+    return det_label.contiguous(), det_length.contiguous(), det_box.contiguous()
+
+
+def track_gate_blocks(table, shapes, det_label, det_length, det_box, num_classes=8, min_points=2, use_lengths=True,
+                      radius_sq=None):
+    """Packed class gate of every scene's (A_s, D_s) block (pcreid_track_gate_blocks).  table: the device state of a track
+    table (TRACK_SLOT_FIELDS / TRACK_SCENE_FIELDS, e.g. models/tracking.py TrackTable); shapes: host (A_s, D_s) per scene,
+    A_s = active tracks (0 for a scene without a frame); det_label / det_length int32 (sum D_s,), det_box f32 (sum D_s, 7)
+    packed over the scenes; radius_sq: None or f32 (num_classes,) squared ground-plane radius per class on the device.
+    -> bool (sum A_s * D_s,), scene s's row-major block after scene s-1's (the packing linear_assignment_blocks reads).
+    Checks shapes on the host and never reads device memory back."""
+    S, C, dev = _track_state(table)
+    shapes, offs, off = _track_offsets(shapes, S, C, dev)
+    det_label, det_length, det_box = _det_arrays(offs[1][-1], det_label, det_length, det_box, dev)
+    if radius_sq is not None and (radius_sq.dtype != torch.float32 or tuple(radius_sq.shape) != (num_classes,)
+                                  or radius_sq.device != dev):
+        raise ValueError(f"radius_sq must be float32 of shape ({num_classes},) on {dev}")
+    gate = torch.empty((offs[2][-1],), device=dev, dtype=torch.bool)
+    _OPS.track_gate_blocks(S, C, max((a for a, _ in shapes), default=0), max((d for _, d in shapes), default=0), off,
+                           table.active, table.label, table.length, table.box, det_label, det_length, det_box,
+                           int(num_classes), int(min_points), int(bool(use_lengths)),
+                           None if radius_sq is None else radius_sq.contiguous(), gate)
+    return gate
+
+
+def track_update(table, shapes, track_for_det, det_label, det_length, det_box, max_age=None, replace_all=False):
+    """One step of the track table's bookkeeping for every scene in one launch (pcreid_track_update): matched tracks, ageing and
+    retirement past max_age (None: never), unmatched detections into the lowest free slots, the next active lists and counts.
+    shapes / det_*: as track_gate_blocks; track_for_det int64 (sum D_s,): position in the scene's active list or -1 (the output
+    of linear_assignment_blocks on the gate).  Updates table in place -> (det_track_id int64 (sum D_s,), -1 for a dropped
+    detection; det_row int32 (sum D_s,): the global table row that receives the detection's observation, -1 if none).
+    Checks shapes on the host and never reads device memory back."""
+    S, C, dev = _track_state(table)
+    shapes, offs, off = _track_offsets(shapes, S, C, dev)
+    n = offs[1][-1]
+    det_label, det_length, det_box = _det_arrays(n, det_label, det_length, det_box, dev)
+    if track_for_det.dtype != torch.int64 or tuple(track_for_det.shape) != (n,) or track_for_det.device != dev:
+        raise ValueError(f"track_for_det must be int64 of shape ({n},) on {dev}")
+    if max_age is not None and int(max_age) < 0:
+        raise ValueError("max_age must be None or >= 0")
+    det_track_id = torch.empty((n,), device=dev, dtype=torch.int64)
+    det_row = torch.empty((n,), device=dev, dtype=torch.int32)
+    _OPS.track_update(S, C, max((d for _, d in shapes), default=0), off, track_for_det.contiguous(), det_label, det_length,
+                      det_box, -1 if max_age is None else int(max_age), int(bool(replace_all)), table.alive,
+                      table.track_id, table.label, table.length, table.age, table.hits, table.box, table.next_id,
+                      table.dropped, table.active, table.count, det_track_id, det_row)
+    return det_track_id, det_row
+
+
+def _rows(src, dst, name):
+    """(n, ...) source rows and (R, ...) table rows of one dtype and row shape -> bytes per row"""
+    if src.dtype != dst.dtype or src.shape[1:] != dst.shape[1:] or src.device != dst.device or not dst.is_contiguous():
+        raise ValueError(f"{name}: rows of {tuple(src.shape[1:])} {src.dtype} into a contiguous table of "
+                         f"{tuple(dst.shape[1:])} {dst.dtype}")
+    return math.prod(dst.shape[1:]) * dst.element_size()
+
+
+def track_scatter(det_row, det_xyz, det_feat, xyz, feat):
+    """xyz[det_row[d]] = det_xyz[d] and feat[det_row[d]] = det_feat[d] for every d with det_row[d] >= 0, in one launch
+    (pcreid_track_scatter); rows are copied as bytes, so any dtype works.  det_row int32 (n,) from track_update."""
+    _need_cuda(det_row, det_xyz, det_feat, xyz, feat)
+    n = det_row.shape[0]
+    if det_row.dtype != torch.int32 or det_row.dim() != 1 or det_xyz.shape[0] != n or det_feat.shape[0] != n:
+        raise ValueError("det_row must be int32 (n,) with one xyz and one feature row per entry")
+    bx, bf = _rows(det_xyz, xyz, "xyz"), _rows(det_feat, feat, "feat")
+    _OPS.track_scatter(n, det_row.contiguous(), bx, det_xyz.contiguous(), xyz, bf, det_feat.contiguous(), feat)
+
+
 def bf16_kmajor_image(w):
     """torch weight (N, K) -> bf16 K-major tcgen05 operand image [K/8][N][8] (uint8 view)."""
     n, kd = w.shape

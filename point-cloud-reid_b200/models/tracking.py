@@ -15,6 +15,13 @@
 * ``MultiScenePointReidentifier`` -- ``step`` over many independent scenes (one bank each) with one front-end pass, one
   encode, one pair-scoring call and one assignment launch for all of them; every scene's result and bank equal those of its
   own ``PointReidentifier.step``.
+* ``score_pair_blocks`` -- the pair-list scorer both multi-scene classes share: one ``match_pairs`` call over the gated pairs
+  of many packed (T_b, D_b) blocks.
+* ``TrackTable`` / ``ReIDTracker`` -- the tracker that keeps its tracks: a device-resident table of S scenes x C slots (ids,
+  labels, ages, hits, last boxes, bank rows) and a step that gates, scores, assigns and updates every scene with one launch
+  of each kernel (kernels.track_gate_blocks / track_update / track_scatter) and no per-scene Python loop over tensors.
+  Retirement after ``max_age`` unmatched steps, a bounded bank and an optional centre-distance gate come with it; motion
+  prediction stays with the caller.
 """
 import torch
 
@@ -69,6 +76,27 @@ def class_gate(det_labels, track_labels, det_lengths=None, track_lengths=None, u
         ok_t = ok_t & (track_lengths >= min_points)
         ok_d = ok_d & (det_lengths >= min_points)
     return (track_labels[:, None] == det_labels[None, :]) & ok_t[:, None] & ok_d[None, :]
+
+
+def score_pair_blocks(model, gate, shapes, det_starts, h_t, xyz_t, h_d, xyz_d):
+    """Logits of the gated pairs of many (T_b, D_b) blocks in one ``model.match_pairs`` call.  gate: bool, block b's row-major
+    (T_b, D_b) mask after block b-1's (the packing of kernels.linear_assignment_blocks); block b's tracks are rows
+    sum_{c<b} T_c .. of h_t / xyz_t, its detections rows det_starts[b] .. of h_d / xyz_d.
+    -> packed float32 cost like gate: the logit where gate is set, 0 elsewhere."""
+    dev = gate.device
+    e_off, t_off = [0], [0]
+    for T, D in shapes:
+        e_off.append(e_off[-1] + T * D)
+        t_off.append(t_off[-1] + T)
+    meta = torch.tensor([e_off[:-1], t_off[:-1], list(det_starts), [D for _, D in shapes]], dtype=torch.int64).to(dev)
+    e = gate.nonzero().squeeze(1)
+    blk = torch.searchsorted(torch.tensor(e_off[1:], dtype=torch.int64).to(dev), e, right=True)
+    local = e - meta[0, blk]
+    ti = meta[1, blk] + local // meta[3, blk]
+    dj = meta[2, blk] + local % meta[3, blk]
+    cost = torch.zeros(gate.shape, device=dev, dtype=torch.float32)
+    cost[e] = model.match_pairs(h_t, xyz_t, h_d, xyz_d, ti, dj)
+    return cost
 
 
 class PointReidentifier:
@@ -217,21 +245,158 @@ class MultiScenePointReidentifier:
             cost = torch.cat([self.model.match_all_pairs(ht, xt, h_d[d0[k]:d0[k + 1]], xyz_d[d0[k]:d0[k + 1]], pair_mask=g).reshape(-1)
                               for (_, k, _, _), g, xt, ht in zip(blocks, gates, xyz_t, h_t)])
             return cost, gate
-        # 4. one match_pairs call over every scene's gated pairs, indices into the concatenated track / detection sets
-        dev = gate.device
-        e_off, t_off, d_off, cols = [0], [0], [], []
-        for _, k, T, D in blocks:
-            e_off.append(e_off[-1] + T * D)
-            t_off.append(t_off[-1] + T)
-            d_off.append(d0[k])
-            cols.append(D)
-        meta = torch.tensor([e_off[:-1], t_off[:-1], d_off, cols], dtype=torch.int64).to(dev)
-        e = gate.nonzero().squeeze(1)
-        blk = torch.searchsorted(torch.tensor(e_off[1:], dtype=torch.int64).to(dev), e, right=True)
-        local = e - meta[0, blk]
-        ti = meta[1, blk] + local // meta[3, blk]
-        dj = meta[2, blk] + local % meta[3, blk]
-        # 5. logits scattered into the packed cost
-        cost = torch.zeros(gate.shape, device=dev, dtype=torch.float32)
-        cost[e] = self.model.match_pairs(torch.cat(h_t), torch.cat(xyz_t), h_d, xyz_d, ti, dj)
+        # 4. one match_pairs call over every scene's gated pairs; 5. logits scattered into the packed cost
+        cost = score_pair_blocks(self.model, gate, [(T, D) for _, _, T, D in blocks], [d0[k] for _, k, _, _ in blocks],
+                                 torch.cat(h_t), torch.cat(xyz_t), h_d, xyz_d)
         return cost, gate
+
+
+class TrackTable:
+    """Tracks of S scenes kept on the device: C slots per scene (1 <= C <= 4096), the state of kernels.TRACK_SLOT_FIELDS /
+    TRACK_SCENE_FIELDS plus the bank rows ``xyz`` / ``feat`` (S * C rows; row r = s * C + slot), allocated from the first
+    encode with its row shapes and dtypes.  A slot holds alive, track_id (unique within its scene, from 0, never reused),
+    label, length (points of the kept observation), age (steps since the last match), hits and box (the last matched
+    detection's 7 box values).  Per scene: next_id, dropped (detections that found no free slot), count and the active list
+    ``active[s, :count[s]]`` (global rows of the alive slots, ascending).  Updated by ReIDTracker.step through
+    kernels.track_update / track_scatter; the observation is replaced on a match when replace_all or when the new one has at
+    least as many points (PointFeatureSet.replace_old's rule)."""
+
+    def __init__(self, num_scenes, capacity, replace_all=False, device="cuda"):
+        if not 1 <= capacity <= K.TRACK_MAX_CAPACITY or not 1 <= num_scenes <= K.TRACK_MAX_SCENES:
+            raise ValueError(f"TrackTable supports 1 <= capacity <= {K.TRACK_MAX_CAPACITY} and 1 <= num_scenes <= "
+                             f"{K.TRACK_MAX_SCENES}; got {(num_scenes, capacity)}")
+        self.num_scenes, self.capacity, self.replace_all = int(num_scenes), int(capacity), bool(replace_all)
+        self.device = torch.device(device)
+        for name, dtype, tail in K.TRACK_SLOT_FIELDS:
+            setattr(self, name, torch.zeros((self.num_scenes, self.capacity) + tail, dtype=dtype, device=self.device))
+        for name, dtype in K.TRACK_SCENE_FIELDS:
+            setattr(self, name, torch.zeros((self.num_scenes,), dtype=dtype, device=self.device))
+        self.xyz = self.feat = None
+
+    def ensure_rows(self, xyz, feat):
+        """allocates the bank rows from the first encode's (n, ...) outputs; later encodes must have the same row shapes"""
+        if self.xyz is None:
+            n = self.num_scenes * self.capacity
+            self.xyz = torch.zeros((n,) + tuple(xyz.shape[1:]), dtype=xyz.dtype, device=self.device)
+            self.feat = torch.zeros((n,) + tuple(feat.shape[1:]), dtype=feat.dtype, device=self.device)
+        elif self.xyz.shape[1:] != xyz.shape[1:] or self.feat.shape[1:] != feat.shape[1:]:
+            raise ValueError(f"encoder rows {tuple(xyz.shape[1:])} / {tuple(feat.shape[1:])} differ from the table's "
+                             f"{tuple(self.xyz.shape[1:])} / {tuple(self.feat.shape[1:])}")
+
+    def tracks(self, s):
+        """-> (ids int64, labels, boxes (n, 7), ages, hits, rows int64 into xyz / feat) of scene s's alive slots, ascending slot
+        order (reads the device: for inspection, not for the step)"""
+        slot = self.alive[s].nonzero().squeeze(1)
+        return (self.track_id[s, slot], self.label[s, slot], self.box[s, slot], self.age[s, slot], self.hits[s, slot],
+                s * self.capacity + slot)
+
+    def reset(self, s):
+        """forgets every track of scene s: ids start again from 0"""
+        for name, _, _ in K.TRACK_SLOT_FIELDS:
+            getattr(self, name)[s].zero_()
+        for name, _ in K.TRACK_SCENE_FIELDS:
+            getattr(self, name)[s] = 0
+
+
+def _to_device(values, dtype, dev):
+    t = torch.tensor(values, dtype=dtype)
+    return t.pin_memory().to(dev, non_blocking=True) if dev.type == "cuda" else t
+
+
+class ReIDTracker:
+    """A tracker over S scenes whose tracks live in a TrackTable: ids, ages, hits, retirement after ``max_age`` unmatched
+    steps (None: never) and a bounded bank of ``capacity`` slots per scene, all updated on the device.
+
+    ``step(frames, min_score, sample_ranks)`` runs, once each for all scenes: the segmented crop front-end, one encode, one
+    gather of every active track's rows, kernels.track_gate_blocks (class_gate's rule, plus ``max_distance`` when given),
+    the pair-list scorer (``'concat'`` models: scene by scene through their dense head), kernels.linear_assignment_blocks,
+    kernels.track_update and kernels.track_scatter.  Its one host read is the S active counts.
+
+    ``max_distance``: None, a float or one float per class; a track and a detection may then only be paired when their box
+    centres are within that distance in the ground plane (x, y), tested in float32 as fl(dx*dx + dy*dy) <= fl(r*r).  That test
+    is only meaningful when the boxes of every step are given in one fixed frame (e.g. world coordinates); the crop only needs
+    each sweep and its boxes to agree.
+
+    With max_age=None, a capacity that never fills and no max_distance, slots are handed out in append order and scene s's
+    table is, row for row, the bank of PointReidentifier.step called with track_index = arange(len(bank)) and the stored
+    labels; a detection's track id is then that bank row."""
+
+    def __init__(self, model, num_scenes=1, capacity=1024, max_age=None, max_distance=None, replace_all=False, use_lengths=True,
+                 num_classes=8, min_points=2, subsample_number=128, device="cuda"):
+        if max_age is not None and max_age < 0:
+            raise ValueError("max_age must be None or >= 0")
+        self.model = model
+        self.table = TrackTable(num_scenes, capacity, replace_all, device)
+        self.max_age, self.use_lengths = max_age, use_lengths
+        self.num_classes, self.min_points, self.subsample_number = num_classes, min_points, subsample_number
+        self.radius_sq = None
+        if max_distance is not None:
+            r = torch.as_tensor(max_distance, dtype=torch.float32).flatten()
+            if r.numel() == 1:
+                r = r.expand(num_classes)
+            if r.numel() != num_classes or bool((r < 0).any()) or bool(r.isnan().any()):
+                raise ValueError(f"max_distance must be one non-negative float or {num_classes} of them")
+            self.radius_sq = (r * r).contiguous().to(self.table.device)
+
+    @torch.no_grad()
+    def step(self, frames, min_score, sample_ranks=None):
+        """frames[s]: (sweep (P, >=3), bboxes (D_s, >=7), det_labels (D_s,)) or None (the scene is frozen: nothing ages);
+        sample_ranks: None (drawn on the device) or one (D_s, N) int64 tensor per scene with a frame.
+        -> per scene (track_id_for_det (D_s,) int64, -1 for a detection that found no free slot; cost (A_s, D_s) logits, 0
+        where not compared, or None when the scene had no active tracks), None for a frozen scene."""
+        tab = self.table
+        S, C, dev = tab.num_scenes, tab.capacity, tab.device
+        if len(frames) != S:
+            raise ValueError(f"{len(frames)} frames for {S} scenes")
+        live = [s for s, f in enumerate(frames) if f is not None]
+        results = [None] * S
+        if not live:
+            return results
+        if sample_ranks is not None and any(sample_ranks[s] is None for s in live):
+            raise ValueError("sample_ranks must give ranks for every scene with a frame, or be None")
+        counts = tab.count.tolist()                                        # the step's one host read
+        sweeps = [frames[s][0].float() for s in live]
+        boxes = [frames[s][1][:, :7].float() for s in live]
+        A, D = [0] * S, [0] * S
+        for k, s in enumerate(live):
+            A[s], D[s] = counts[s], boxes[k].shape[0]
+        shapes = list(zip(A, D))
+        # 1. crop / centre / resample every scene's detections from its own sweep; 2. one encode
+        rank = None if sample_ranks is None else torch.cat([sample_ranks[s].to(sweeps[0].device, torch.int64) for s in live])
+        det_points, det_len = crop_center_resample_scenes(torch.cat(boxes), torch.cat([w[:, :3] for w in sweeps]),
+                                                          [D[s] for s in live], [w.shape[0] for w in sweeps],
+                                                          self.subsample_number, sample_rank=rank)
+        xyz_d, h_d = self.model.encode(det_points)
+        tab.ensure_rows(xyz_d, h_d)
+        det_label = torch.cat([frames[s][2] for s in live]).to(dev, torch.int32)
+        det_length = det_len.to(dev, torch.int32)
+        det_box = torch.cat(boxes).to(dev).contiguous()
+        # 3. one gather of the rows of every scene's active tracks
+        rows = tab.active.view(-1)[_to_device([s * C + i for s in range(S) for i in range(A[s])], torch.int64, dev)].long()
+        xyz_t, h_t = tab.xyz[rows], tab.feat[rows]
+        # 4. the gate of every scene's (A_s, D_s) block
+        gate = K.track_gate_blocks(tab, shapes, det_label, det_length, det_box, self.num_classes, self.min_points,
+                                   self.use_lengths, self.radius_sq)
+        d0, t0, e0 = [0], [0], [0]
+        for a, d in shapes:
+            d0.append(d0[-1] + d)
+            t0.append(t0[-1] + a)
+            e0.append(e0[-1] + a * d)
+        # 5. the logits of the gated pairs
+        if gate.numel() == 0:
+            cost = torch.zeros((0,), device=dev, dtype=torch.float32)
+        elif self.model.match_type == 'concat':
+            cost = torch.cat([self.model.match_all_pairs(h_t[t0[s]:t0[s + 1]], xyz_t[t0[s]:t0[s + 1]], h_d[d0[s]:d0[s + 1]],
+                                                         xyz_d[d0[s]:d0[s + 1]],
+                                                         pair_mask=gate[e0[s]:e0[s + 1]].view(a, d)).reshape(-1)
+                              for s, (a, d) in enumerate(shapes) if a * d])
+        else:
+            cost = score_pair_blocks(self.model, gate, shapes, d0[:-1], h_t, xyz_t, h_d, xyz_d)
+        # 6. one assignment launch; 7. the table's bookkeeping; 8. the stored observations into their rows
+        _, track_for_det = K.linear_assignment_blocks(cost, shapes, min_score, gate)
+        det_track_id, det_row = K.track_update(tab, shapes, track_for_det, det_label, det_length, det_box, self.max_age,
+                                               tab.replace_all)
+        K.track_scatter(det_row, xyz_d, h_d, tab.xyz, tab.feat)
+        for s in live:
+            results[s] = (det_track_id[d0[s]:d0[s + 1]], cost[e0[s]:e0[s + 1]].view(A[s], D[s]) if A[s] else None)
+        return results

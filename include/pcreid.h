@@ -325,6 +325,37 @@ int pcreid_track_update(int S, int C, int max_D, const long long* offsets, const
 int pcreid_track_scatter(int n_det, const int* det_row, long long xyz_bytes, const void* det_xyz, void* xyz,
                          long long feat_bytes, const void* det_feat, void* feat, void* stream);
 
+/* Motion of the track table: a constant-velocity Kalman filter per slot (AB3DMOT's model).  State: kf_box (S * C, 7) f32, the
+ * box estimate (x, y, z, dx, dy, dz, yaw); kf_vel (S * C, 3) f32, (vx, vy, vz) per unit of dt; kf_cov (S * C, 13) f32, the
+ * covariance, exact in 13 values because F is constant velocity, H selects the box and Q, R and P0 are diagonal:
+ * [3a, 3a + 1, 3a + 2] = (P_pp, P_pv, P_vv) of axis a in {x, y, z}, [9 .. 12] = the variances of dx, dy, dz and yaw.
+ * Offsets, size limits and error codes as pcreid_track_*; all arithmetic f32, one rounding per operation in the order below;
+ * TWO_PI = fl(2 pi), wrap(a) = a - TWO_PI * rint(a / TWO_PI); q, q_vel >= 0 and init_var, init_vel_var, r > 0, finite.
+ *
+ * pcreid_track_predict: for track i < A_s of scene s (row active[s * C + i]), dt (S,) f32 on the device, per axis:
+ *   p += dt*v;  t = P_pv + dt*P_vv;  P_pp = P_pp + dt*(P_pv + t) + q;  P_pv = t;  P_vv += q_vel;  the other four variances + q.
+ * pcreid_track_correct, after pcreid_track_update of the same step: track_rows (sum A_s) int64 = the active rows entering the
+ *   step, packed by scene at offsets[0] (NULL allowed when every A_s is 0).  Detection d with track_for_det[d] >= 0 corrects
+ *   row track_rows[offsets[0][s] + track_for_det[d]] with z = det_box[d]: per axis s = P_pp + r; kp = P_pp/s; kv = P_pv/s;
+ *   y = z - p; p += kp*y; v += kv*y; P_vv -= kv*P_pv; P_pv = kv*r; P_pp = kp*r (the last three from the pre-update values);
+ *   dx, dy, dz: k = P/(P + r); b += k*(z - b); P = k*r; yaw: k as for the sizes, y = wrap(z - yaw), y = wrap(y + fl(pi)) when
+ *   |y| > fl(pi/2) (flipped heading), yaw = wrap(yaw + k*y), P = k*r.  Detection d with track_for_det[d] < 0 and
+ *   det_row[d] >= 0 is born at det_row[d]: box = d's box with wrap(yaw), velocity 0, covariance (init_var, 0, init_vel_var)
+ *   per axis and init_var for the other four.  A dropped detection (det_row -1) changes nothing.
+ * pcreid_track_gate_motion_blocks: pcreid_track_gate_blocks with box = kf_box (the predicted boxes); when gate_chi2 > 0 a
+ *   pair also needs fl(fl(fl(dx*dx)/Sx) + fl(fl(dy*dy)/Sy)) <= gate_chi2, Sx = fl(kf_cov[0] + r), Sy = fl(kf_cov[3] + r)
+ *   (the Mahalanobis distance of the ground-plane innovation); gate_chi2 <= 0: no such bound (kf_cov may be NULL). */
+int pcreid_track_predict(int S, int C, int max_A, const long long* offsets, const int* active, const float* dt, float* kf_box,
+                         float* kf_vel, float* kf_cov, float q, float q_vel, void* stream);
+int pcreid_track_correct(int S, int C, int max_D, const long long* offsets, const long long* track_rows,
+                         const long long* track_for_det, const float* det_box, const int* det_row, float* kf_box, float* kf_vel,
+                         float* kf_cov, float init_var, float init_vel_var, float r, void* stream);
+int pcreid_track_gate_motion_blocks(int S, int C, int max_A, int max_D, const long long* offsets, const int* active,
+                                    const int* label, const int* length, const float* box, const int* det_label,
+                                    const int* det_length, const float* det_box, int num_classes, int min_points, int use_lengths,
+                                    const float* r2, const float* kf_cov, float r, float gate_chi2, unsigned char* gate,
+                                    void* stream);
+
 /* ------------------------------------------------------------------ B'. fused tensor-core match path --- */
 /* Tensor-core modes of the xcorr_eff head (csrc/pair_tc.cu, csrc/pair_tc2.cu): tcgen05 kind::f16 GEMMs with fp32
  * accumulation and fp32 norms.  `fmt` selects the 16-bit operand format of EVERY operand image of a call chain:

@@ -105,6 +105,9 @@ _SIGS = {
     "pcreid_track_gate_blocks": [c_int] * 4 + [c_vp] * 8 + [c_int] * 3 + [c_vp, c_vp, c_vp],
     "pcreid_track_update": [c_int] * 3 + [c_vp] * 5 + [c_int, c_int] + [c_vp] * 13 + [c_vp],
     "pcreid_track_scatter": [c_int, c_vp, c_ll, c_vp, c_vp, c_ll, c_vp, c_vp, c_vp],
+    "pcreid_track_predict": [c_int] * 3 + [c_vp] * 6 + [c_float, c_float, c_vp],
+    "pcreid_track_correct": [c_int] * 3 + [c_vp] * 8 + [c_float] * 3 + [c_vp],
+    "pcreid_track_gate_motion_blocks": [c_int] * 4 + [c_vp] * 8 + [c_int] * 3 + [c_vp, c_vp, c_float, c_float, c_vp, c_vp],
 }
 
 ERRORS = {1: "PCREID_ERR_ARG (bad pointer/size)", 2: "PCREID_ERR_LAUNCH (CUDA launch failed)",

@@ -10,9 +10,16 @@
 //                           then the next active list.  Ranks come from block-wide scans over contiguous per-thread ranges,
 //                           so they are in slot / detection order whatever the thread count.
 // pcreid_track_scatter:     the stored detections' xyz / feature rows (opaque bytes) into their table rows.
+//
+// Motion (constant-velocity Kalman filter per slot, the compact covariance of include/pcreid.h), one thread per track or
+// detection, f32 without contraction so that the CPU restatement reproduces it bit for bit:
+// pcreid_track_predict:            every active track of a scene with a frame, by that scene's dt.
+// pcreid_track_correct:            after pcreid_track_update: matched tracks take their detection, newborn slots start.
+// pcreid_track_gate_motion_blocks: pcreid_track_gate_blocks' gate on the predicted boxes, plus a Mahalanobis bound.
 #include "../../include/pcreid.h"
 #include "common.cuh"
 
+#include <cmath>
 #include <cstdint>
 
 namespace {
@@ -23,6 +30,56 @@ constexpr int UPDATE_THREADS = 512;
 constexpr int GATE_THREADS = 256;
 constexpr int SCATTER_THREADS = 256;
 constexpr long long SCATTER_CHUNK = SCATTER_THREADS * 16 * 4;   // bytes of one row one CTA copies
+
+constexpr int MOTION_THREADS = 256;
+constexpr int COV = 13;                  // the compact covariance of one slot (include/pcreid.h)
+constexpr float TWO_PI = 6.28318548f;    // fl(2 pi) = 2 fl(pi)
+constexpr float PI_F = 3.14159274f;      // fl(pi)
+constexpr float HALF_PI = 1.57079637f;   // fl(pi / 2)
+
+// the gate of table row r and detection j.  cov == nullptr: class rule and radius only (pcreid_track_gate_blocks); else the
+// ground-plane Mahalanobis bound as well.  No contraction: the CPU restatement reproduces this bit for bit.
+__device__ __forceinline__ bool gate_pair(long long r, long long j, const int* __restrict__ label,
+                                          const int* __restrict__ length, const float* __restrict__ box,
+                                          const int* __restrict__ det_label, const int* __restrict__ det_length,
+                                          const float* __restrict__ det_box, int num_classes, int min_points, int use_lengths,
+                                          const float* __restrict__ r2, const float* __restrict__ cov, float meas_var,
+                                          float chi2) {
+  const int lt = label[r];
+  bool ok = lt == det_label[j] && lt >= 0 && lt < num_classes;
+  if (use_lengths) ok = ok && length[r] >= min_points && det_length[j] >= min_points;
+  if (ok && (r2 || cov)) {
+    const float dx = __fsub_rn(box[r * 7], det_box[j * 7]), dy = __fsub_rn(box[r * 7 + 1], det_box[j * 7 + 1]);
+    if (r2) ok = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)) <= r2[lt];
+    if (ok && cov) {
+      const float sx = __fadd_rn(cov[r * COV], meas_var), sy = __fadd_rn(cov[r * COV + 3], meas_var);
+      ok = __fadd_rn(__fdiv_rn(__fmul_rn(dx, dx), sx), __fdiv_rn(__fmul_rn(dy, dy), sy)) <= chi2;
+    }
+  }
+  return ok;
+}
+
+// the packed gate of scene blockIdx.y's (A_s, D_s) block, grid-stride over its elements; both gate kernels are this loop
+__device__ __forceinline__ void gate_blocks(int S, int C, const long long* __restrict__ off, const int* __restrict__ active,
+                                            const int* __restrict__ label, const int* __restrict__ length,
+                                            const float* __restrict__ box, const int* __restrict__ det_label,
+                                            const int* __restrict__ det_length, const float* __restrict__ det_box,
+                                            int num_classes, int min_points, int use_lengths, const float* __restrict__ r2,
+                                            const float* __restrict__ cov, float meas_var, float chi2,
+                                            unsigned char* __restrict__ gate) {
+  const int s = blockIdx.y;
+  const int A = (int)(off[s + 1] - off[s]);
+  const int D = (int)(off[(S + 1) + s + 1] - off[(S + 1) + s]);
+  const long long d0 = off[(S + 1) + s], e0 = off[2 * (S + 1) + s];
+  const long long n = (long long)A * D;
+  const int* act = active + (long long)s * C;
+  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+    const int i = (int)(e / D);
+    const long long j = d0 + (e - (long long)i * D);
+    gate[e0 + e] = gate_pair(act[i], j, label, length, box, det_label, det_length, det_box, num_classes, min_points, use_lengths,
+                             r2, cov, meas_var, chi2) ? 1 : 0;
+  }
+}
 
 __global__ void __launch_bounds__(GATE_THREADS) track_gate_kernel(int S, int C, const long long* __restrict__ off,
                                                                    const int* __restrict__ active,
@@ -35,26 +92,108 @@ __global__ void __launch_bounds__(GATE_THREADS) track_gate_kernel(int S, int C, 
                                                                    int min_points, int use_lengths,
                                                                    const float* __restrict__ r2,
                                                                    unsigned char* __restrict__ gate) {
+  gate_blocks(S, C, off, active, label, length, box, det_label, det_length, det_box, num_classes, min_points, use_lengths, r2,
+              nullptr, 0.f, 0.f, gate);
+}
+
+// pcreid_track_gate_motion_blocks: track_gate_kernel on the predicted boxes, plus the Mahalanobis bound when cov != nullptr
+__global__ void __launch_bounds__(GATE_THREADS) track_gate_motion_kernel(
+    int S, int C, const long long* __restrict__ off, const int* __restrict__ active, const int* __restrict__ label,
+    const int* __restrict__ length, const float* __restrict__ box, const int* __restrict__ det_label,
+    const int* __restrict__ det_length, const float* __restrict__ det_box, int num_classes, int min_points, int use_lengths,
+    const float* __restrict__ r2, const float* __restrict__ cov, float meas_var, float chi2, unsigned char* __restrict__ gate) {
+  gate_blocks(S, C, off, active, label, length, box, det_label, det_length, det_box, num_classes, min_points, use_lengths, r2,
+              cov, meas_var, chi2, gate);
+}
+
+__device__ __forceinline__ float wrap_angle(float a) {
+  return __fsub_rn(a, __fmul_rn(TWO_PI, rintf(__fdiv_rn(a, TWO_PI))));
+}
+
+// thread (x, s): track i of scene s (row active[s * C + i]) moves by dt[s] * velocity; its covariance grows
+__global__ void __launch_bounds__(MOTION_THREADS) track_predict_kernel(int S, int C, const long long* __restrict__ off,
+                                                                        const int* __restrict__ active,
+                                                                        const float* __restrict__ dt_s, float* __restrict__ kf_box,
+                                                                        float* __restrict__ kf_vel, float* __restrict__ kf_cov,
+                                                                        float q, float q_vel) {
   const int s = blockIdx.y;
   const int A = (int)(off[s + 1] - off[s]);
-  const int D = (int)(off[(S + 1) + s + 1] - off[(S + 1) + s]);
-  const long long d0 = off[(S + 1) + s], e0 = off[2 * (S + 1) + s];
-  const long long n = (long long)A * D;
-  const int* act = active + (long long)s * C;
-  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
-    const int i = (int)(e / D);
-    const long long j = d0 + (e - (long long)i * D);
-    const long long r = act[i];
-    const int lt = label[r];
-    bool ok = lt == det_label[j] && lt >= 0 && lt < num_classes;
-    if (use_lengths) ok = ok && length[r] >= min_points && det_length[j] >= min_points;
-    if (ok && r2) {
-      // no contraction: the CPU restatement reproduces this bit for bit
-      const float dx = __fsub_rn(box[r * 7], det_box[j * 7]), dy = __fsub_rn(box[r * 7 + 1], det_box[j * 7 + 1]);
-      ok = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)) <= r2[lt];
-    }
-    gate[e0 + e] = ok ? 1 : 0;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= A) return;
+  const long long r = active[(long long)s * C + i];
+  const float dt = dt_s[s];
+  float* b = kf_box + r * 7;
+  float* P = kf_cov + r * COV;
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    const float v = kf_vel[r * 3 + a];
+    const float pp = P[3 * a], pv = P[3 * a + 1], vv = P[3 * a + 2];
+    b[a] = __fadd_rn(b[a], __fmul_rn(dt, v));
+    const float t = __fadd_rn(pv, __fmul_rn(dt, vv));
+    P[3 * a] = __fadd_rn(__fadd_rn(pp, __fmul_rn(dt, __fadd_rn(pv, t))), q);
+    P[3 * a + 1] = t;
+    P[3 * a + 2] = __fadd_rn(vv, q_vel);
   }
+#pragma unroll
+  for (int k = 9; k < COV; ++k) P[k] = __fadd_rn(P[k], q);
+}
+
+// thread (x, s): detection d of scene s corrects its matched track, or initialises the slot it was born into
+__global__ void __launch_bounds__(MOTION_THREADS) track_correct_kernel(
+    int S, const long long* __restrict__ off, const long long* __restrict__ track_rows, const long long* __restrict__ track_for_det,
+    const float* __restrict__ det_box, const int* __restrict__ det_row, float* __restrict__ kf_box, float* __restrict__ kf_vel,
+    float* __restrict__ kf_cov, float init_var, float init_vel_var, float meas_var) {
+  const int s = blockIdx.y;
+  const int D = (int)(off[(S + 1) + s + 1] - off[(S + 1) + s]);
+  const int d = blockIdx.x * blockDim.x + threadIdx.x;
+  if (d >= D) return;
+  const long long j = off[(S + 1) + s] + d;
+  const long long t = track_for_det[j];
+  const float* z = det_box + j * 7;
+  if (t < 0) {
+    const long long r = det_row[j];
+    if (r < 0) return;                                   // dropped: no slot
+#pragma unroll
+    for (int k = 0; k < 6; ++k) kf_box[r * 7 + k] = z[k];
+    kf_box[r * 7 + 6] = wrap_angle(z[6]);
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      kf_vel[r * 3 + a] = 0.f;
+      kf_cov[r * COV + 3 * a] = init_var;
+      kf_cov[r * COV + 3 * a + 1] = 0.f;
+      kf_cov[r * COV + 3 * a + 2] = init_vel_var;
+    }
+#pragma unroll
+    for (int k = 9; k < COV; ++k) kf_cov[r * COV + k] = init_var;
+    return;
+  }
+  const long long r = track_rows[off[s] + t];
+  float* b = kf_box + r * 7;
+  float* P = kf_cov + r * COV;
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    const float pp = P[3 * a], pv = P[3 * a + 1], vv = P[3 * a + 2];
+    const float sa = __fadd_rn(pp, meas_var);
+    const float kp = __fdiv_rn(pp, sa), kv = __fdiv_rn(pv, sa);
+    const float y = __fsub_rn(z[a], b[a]);
+    b[a] = __fadd_rn(b[a], __fmul_rn(kp, y));
+    kf_vel[r * 3 + a] = __fadd_rn(kf_vel[r * 3 + a], __fmul_rn(kv, y));
+    P[3 * a + 2] = __fsub_rn(vv, __fmul_rn(kv, pv));
+    P[3 * a + 1] = __fmul_rn(kv, meas_var);
+    P[3 * a] = __fmul_rn(kp, meas_var);
+  }
+#pragma unroll
+  for (int a = 3; a < 6; ++a) {
+    const float k = __fdiv_rn(P[6 + a], __fadd_rn(P[6 + a], meas_var));
+    b[a] = __fadd_rn(b[a], __fmul_rn(k, __fsub_rn(z[a], b[a])));
+    P[6 + a] = __fmul_rn(k, meas_var);
+  }
+  // yaw: the innovation wrapped to (-pi, pi], and turned by pi when the detection's heading is flipped (AB3DMOT)
+  const float k = __fdiv_rn(P[12], __fadd_rn(P[12], meas_var));
+  float y = wrap_angle(__fsub_rn(z[6], b[6]));
+  if (fabsf(y) > HALF_PI) y = wrap_angle(__fadd_rn(y, PI_F));
+  b[6] = wrap_angle(__fadd_rn(b[6], __fmul_rn(k, y)));
+  P[12] = __fmul_rn(k, meas_var);
 }
 
 // exclusive prefix of v over the CTA in thread order; *total = the sum.  Every thread calls it; sh holds 32 ints.
@@ -236,6 +375,54 @@ int pcreid_track_gate_blocks(int S, int C, int max_A, int max_D, const long long
   track_gate_kernel<<<dim3(gx, S), GATE_THREADS, 0, (cudaStream_t)stream>>>(S, C, offsets, active, label, length, box, det_label,
                                                                             det_length, det_box, num_classes, min_points,
                                                                             use_lengths, r2, gate);
+  return pcreid_launch_status();
+}
+
+int pcreid_track_gate_motion_blocks(int S, int C, int max_A, int max_D, const long long* offsets, const int* active,
+                                    const int* label, const int* length, const float* box, const int* det_label,
+                                    const int* det_length, const float* det_box, int num_classes, int min_points, int use_lengths,
+                                    const float* r2, const float* kf_cov, float r, float gate_chi2, unsigned char* gate,
+                                    void* stream) {
+  if (S < 0 || C < 1 || max_A < 0 || max_D < 0 || max_A > C || num_classes < 0) return PCREID_ERR_ARG;
+  if (!(isfinite(gate_chi2) && isfinite(r))) return PCREID_ERR_ARG;
+  const bool chi2 = gate_chi2 > 0.f;
+  if (chi2 && !(r > 0.f)) return PCREID_ERR_ARG;
+  if (S > MAX_SCENES || C > TRACK_MAX || max_D > TRACK_MAX) return PCREID_ERR_UNSUPPORTED;
+  if (S == 0 || max_A == 0 || max_D == 0) return PCREID_OK;
+  if (!offsets || !active || !label || !det_label || !gate || (use_lengths && (!length || !det_length)) ||
+      ((r2 || chi2) && (!box || !det_box)) || (chi2 && !kf_cov))
+    return PCREID_ERR_ARG;
+  const long long per_scene = (long long)max_A * max_D;
+  const int gx = (int)min((per_scene + GATE_THREADS - 1) / GATE_THREADS, 1024LL);
+  track_gate_motion_kernel<<<dim3(gx, S), GATE_THREADS, 0, (cudaStream_t)stream>>>(
+      S, C, offsets, active, label, length, box, det_label, det_length, det_box, num_classes, min_points, use_lengths, r2,
+      chi2 ? kf_cov : nullptr, r, gate_chi2, gate);
+  return pcreid_launch_status();
+}
+
+int pcreid_track_predict(int S, int C, int max_A, const long long* offsets, const int* active, const float* dt, float* kf_box,
+                         float* kf_vel, float* kf_cov, float q, float q_vel, void* stream) {
+  if (S < 0 || C < 1 || max_A < 0 || max_A > C) return PCREID_ERR_ARG;
+  if (!(isfinite(q) && q >= 0.f && isfinite(q_vel) && q_vel >= 0.f)) return PCREID_ERR_ARG;
+  if (S > MAX_SCENES || C > TRACK_MAX) return PCREID_ERR_UNSUPPORTED;
+  if (S == 0 || max_A == 0) return PCREID_OK;
+  if (!offsets || !active || !dt || !kf_box || !kf_vel || !kf_cov) return PCREID_ERR_ARG;
+  track_predict_kernel<<<dim3((max_A + MOTION_THREADS - 1) / MOTION_THREADS, S), MOTION_THREADS, 0, (cudaStream_t)stream>>>(
+      S, C, offsets, active, dt, kf_box, kf_vel, kf_cov, q, q_vel);
+  return pcreid_launch_status();
+}
+
+int pcreid_track_correct(int S, int C, int max_D, const long long* offsets, const long long* track_rows,
+                         const long long* track_for_det, const float* det_box, const int* det_row, float* kf_box, float* kf_vel,
+                         float* kf_cov, float init_var, float init_vel_var, float r, void* stream) {
+  if (S < 0 || C < 1 || max_D < 0) return PCREID_ERR_ARG;
+  if (!(isfinite(init_var) && init_var > 0.f && isfinite(init_vel_var) && init_vel_var > 0.f && isfinite(r) && r > 0.f))
+    return PCREID_ERR_ARG;
+  if (S > MAX_SCENES || C > TRACK_MAX || max_D > TRACK_MAX) return PCREID_ERR_UNSUPPORTED;
+  if (S == 0 || max_D == 0) return PCREID_OK;
+  if (!offsets || !track_for_det || !det_box || !det_row || !kf_box || !kf_vel || !kf_cov) return PCREID_ERR_ARG;
+  track_correct_kernel<<<dim3((max_D + MOTION_THREADS - 1) / MOTION_THREADS, S), MOTION_THREADS, 0, (cudaStream_t)stream>>>(
+      S, offsets, track_rows, track_for_det, det_box, det_row, kf_box, kf_vel, kf_cov, init_var, init_vel_var, r);
   return pcreid_launch_status();
 }
 

@@ -716,6 +716,105 @@ def track_update(table, shapes, track_for_det, det_label, det_length, det_box, m
     return det_track_id, det_row
 
 
+# the motion state of a track table built with motion (models/tracking.py, MotionModel): the constant-velocity Kalman filter's
+# box estimate, velocity and compact covariance per slot (layout: include/pcreid.h, pcreid_track_predict)
+TRACK_MOTION_FIELDS = (("kf_box", torch.float32, (7,)), ("kf_vel", torch.float32, (3,)), ("kf_cov", torch.float32, (13,)))
+
+
+def _track_motion_state(table, S, C, dev):
+    for name, dtype, tail in TRACK_MOTION_FIELDS:
+        t = getattr(table, name, None)
+        if t is None or t.dtype != dtype or tuple(t.shape) != (S, C) + tail or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"table.{name} must be contiguous {dtype} of shape {(S, C) + tail} on {dev} (a table with motion)")
+
+
+def _finite_scalars(**kw):
+    for name, (v, positive) in kw.items():
+        if isinstance(v, torch.Tensor):
+            raise TypeError(f"{name} must be a Python number (reading a tensor would synchronise)")
+        v = float(v)
+        if not math.isfinite(v) or v < 0 or (positive and v == 0):
+            raise ValueError(f"{name} must be finite and {'> 0' if positive else '>= 0'}; got {v}")
+
+
+def track_dt(dt, S, frozen=()):
+    """a float or one value per scene -> S floats, each finite and >= 0; the entries of the scenes listed in frozen (which
+    are not predicted) are not read and become 0.0"""
+    try:
+        dt = list(dt)
+    except TypeError:
+        dt = [dt] * S
+    if len(dt) != S:
+        raise ValueError(f"{len(dt)} dt values for {S} scenes")
+    frozen = set(frozen)
+    dt = [0.0 if s in frozen else v for s, v in enumerate(dt)]
+    _finite_scalars(**{f"dt[{s}]": (v, False) for s, v in enumerate(dt)})
+    return [float(v) for v in dt]
+
+
+def track_predict(table, shapes, dt, q=1.0, q_vel=0.01):
+    """Kalman prediction of every active track of every scene in one launch (pcreid_track_predict): box += dt * velocity and
+    the covariance grows by the process noise q (box values) / q_vel (velocity).  shapes: host (A_s, D_s) per scene as
+    track_gate_blocks (a scene without a frame has A_s = 0 and is not predicted); dt: host float or one per scene, each finite
+    and >= 0, sent as float32 through pinned memory.  Updates table.kf_box / kf_vel / kf_cov in place.  Checks on the host and
+    never reads device memory back."""
+    S, C, dev = _track_state(table)
+    _track_motion_state(table, S, C, dev)
+    shapes, offs, off = _track_offsets(shapes, S, C, dev)
+    _finite_scalars(q=(q, False), q_vel=(q_vel, False))
+    dt = torch.tensor(track_dt(dt, S), dtype=torch.float32).pin_memory().to(dev, non_blocking=True)
+    _OPS.track_predict(S, C, max((a for a, _ in shapes), default=0), off, table.active, dt, table.kf_box, table.kf_vel,
+                       table.kf_cov, float(q), float(q_vel))
+
+
+def track_correct(table, shapes, track_rows, track_for_det, det_box, det_row, init_var=10.0, init_vel_var=1e4, r=1.0):
+    """Kalman correction after track_update of the same step, every scene in one launch (pcreid_track_correct): a matched
+    detection corrects its track with its box (measurement noise r; yaw with AB3DMOT's flipped-heading rule), an unmatched one
+    that received a slot starts that slot's filter (box, velocity 0, covariance init_var / init_vel_var); a dropped one changes
+    nothing.  shapes / det_box: as track_update; track_rows int64 (sum A_s,): the active rows entering the step, packed by scene
+    (table.active before track_update); track_for_det int64 and det_row int32 (sum D_s,): the inputs and the output of
+    track_update.  Updates table.kf_box / kf_vel / kf_cov in place.  Checks on the host and never reads device memory back."""
+    S, C, dev = _track_state(table)
+    _track_motion_state(table, S, C, dev)
+    shapes, offs, off = _track_offsets(shapes, S, C, dev)
+    _finite_scalars(init_var=(init_var, True), init_vel_var=(init_vel_var, True), r=(r, True))
+    n = offs[1][-1]
+    for name, t, dtype, shape in (("track_rows", track_rows, torch.int64, (offs[0][-1],)),
+                                  ("track_for_det", track_for_det, torch.int64, (n,)),
+                                  ("det_box", det_box, torch.float32, (n, 7)), ("det_row", det_row, torch.int32, (n,))):
+        if t.dtype != dtype or tuple(t.shape) != shape or t.device != dev:
+            raise ValueError(f"{name} must be {dtype} of shape {shape} on {dev}")
+    _OPS.track_correct(S, C, max((d for _, d in shapes), default=0), off, track_rows.contiguous() if track_rows.numel() else None,
+                       track_for_det.contiguous(), det_box.contiguous(), det_row.contiguous(), table.kf_box, table.kf_vel,
+                       table.kf_cov, float(init_var), float(init_vel_var), float(r))
+
+
+def track_gate_motion_blocks(table, shapes, det_label, det_length, det_box, num_classes=8, min_points=2, use_lengths=True,
+                             radius_sq=None, r=1.0, gate_chi2=None):
+    """track_gate_blocks on the predicted boxes (table.kf_box, after track_predict) of a table with motion
+    (pcreid_track_gate_motion_blocks): class_gate's rule, radius_sq around the predicted centre, and when gate_chi2 is given
+    fl(dx*dx / Sx + dy*dy / Sy) <= gate_chi2 with Sx, Sy = the x / y position variance + r (the Mahalanobis distance of the
+    ground-plane innovation).  -> bool (sum A_s * D_s,) packed as track_gate_blocks.  Checks on the host and never reads device
+    memory back."""
+    S, C, dev = _track_state(table)
+    _track_motion_state(table, S, C, dev)
+    shapes, offs, off = _track_offsets(shapes, S, C, dev)
+    det_label, det_length, det_box = _det_arrays(offs[1][-1], det_label, det_length, det_box, dev)
+    if radius_sq is not None and (radius_sq.dtype != torch.float32 or tuple(radius_sq.shape) != (num_classes,)
+                                  or radius_sq.device != dev):
+        raise ValueError(f"radius_sq must be float32 of shape ({num_classes},) on {dev}")
+    _finite_scalars(r=(r, True))
+    if gate_chi2 is not None:
+        _finite_scalars(gate_chi2=(gate_chi2, True))
+    gate = torch.empty((offs[2][-1],), device=dev, dtype=torch.bool)
+    _OPS.track_gate_motion_blocks(S, C, max((a for a, _ in shapes), default=0), max((d for _, d in shapes), default=0), off,
+                                  table.active, table.label, table.length, table.kf_box, det_label, det_length, det_box,
+                                  int(num_classes), int(min_points), int(bool(use_lengths)),
+                                  None if radius_sq is None else radius_sq.contiguous(), table.kf_cov, float(r),
+                                  0.0 if gate_chi2 is None else float(gate_chi2), gate)
+    return gate
+
+
 def _rows(src, dst, name):
     """(n, ...) source rows and (R, ...) table rows of one dtype and row shape -> bytes per row"""
     if src.dtype != dst.dtype or src.shape[1:] != dst.shape[1:] or src.device != dst.device or not dst.is_contiguous():

@@ -20,9 +20,13 @@
 * ``TrackTable`` / ``ReIDTracker`` -- the tracker that keeps its tracks: a device-resident table of S scenes x C slots (ids,
   labels, ages, hits, last boxes, bank rows) and a step that gates, scores, assigns and updates every scene with one launch
   of each kernel (kernels.track_gate_blocks / track_update / track_scatter) and no per-scene Python loop over tensors.
-  Retirement after ``max_age`` unmatched steps, a bounded bank and an optional centre-distance gate come with it; motion
-  prediction stays with the caller.
+  Retirement after ``max_age`` unmatched steps, a bounded bank and an optional centre-distance gate come with it.
+* ``MotionModel`` -- optional motion for ``ReIDTracker``: a constant-velocity Kalman filter per slot in the style of AB3DMOT,
+  kept in the table (kernels.track_predict / track_correct).  Every active track is predicted before the gate, which then
+  tests the predicted box (``max_distance``) and, optionally, the Mahalanobis distance of the predicted ground-plane centre.
 """
+import math
+
 import torch
 
 from .. import kernels as K
@@ -259,15 +263,19 @@ class TrackTable:
     detection's 7 box values).  Per scene: next_id, dropped (detections that found no free slot), count and the active list
     ``active[s, :count[s]]`` (global rows of the alive slots, ascending).  Updated by ReIDTracker.step through
     kernels.track_update / track_scatter; the observation is replaced on a match when replace_all or when the new one has at
-    least as many points (PointFeatureSet.replace_old's rule)."""
+    least as many points (PointFeatureSet.replace_old's rule).
 
-    def __init__(self, num_scenes, capacity, replace_all=False, device="cuda"):
+    With ``motion=True`` each slot also holds the state of kernels.TRACK_MOTION_FIELDS: the Kalman filter's box estimate
+    ``kf_box``, velocity ``kf_vel`` and compact covariance ``kf_cov`` (include/pcreid.h), read with ``motion(s)``."""
+
+    def __init__(self, num_scenes, capacity, replace_all=False, device="cuda", motion=False):
         if not 1 <= capacity <= K.TRACK_MAX_CAPACITY or not 1 <= num_scenes <= K.TRACK_MAX_SCENES:
             raise ValueError(f"TrackTable supports 1 <= capacity <= {K.TRACK_MAX_CAPACITY} and 1 <= num_scenes <= "
                              f"{K.TRACK_MAX_SCENES}; got {(num_scenes, capacity)}")
         self.num_scenes, self.capacity, self.replace_all = int(num_scenes), int(capacity), bool(replace_all)
         self.device = torch.device(device)
-        for name, dtype, tail in K.TRACK_SLOT_FIELDS:
+        self.has_motion = bool(motion)
+        for name, dtype, tail in K.TRACK_SLOT_FIELDS + (K.TRACK_MOTION_FIELDS if self.has_motion else ()):
             setattr(self, name, torch.zeros((self.num_scenes, self.capacity) + tail, dtype=dtype, device=self.device))
         for name, dtype in K.TRACK_SCENE_FIELDS:
             setattr(self, name, torch.zeros((self.num_scenes,), dtype=dtype, device=self.device))
@@ -290,9 +298,17 @@ class TrackTable:
         return (self.track_id[s, slot], self.label[s, slot], self.box[s, slot], self.age[s, slot], self.hits[s, slot],
                 s * self.capacity + slot)
 
+    def motion(self, s):
+        """-> (box estimate (n, 7), velocity (n, 3) per unit of dt) of scene s's alive slots, ascending slot order, as tracks(s)
+        lists them; after a step with motion the box estimate is the corrected one (reads the device: for inspection)"""
+        if not self.has_motion:
+            raise ValueError("this table keeps no motion state (TrackTable(..., motion=True))")
+        slot = self.alive[s].nonzero().squeeze(1)
+        return self.kf_box[s, slot], self.kf_vel[s, slot]
+
     def reset(self, s):
         """forgets every track of scene s: ids start again from 0"""
-        for name, _, _ in K.TRACK_SLOT_FIELDS:
+        for name, _, _ in K.TRACK_SLOT_FIELDS + (K.TRACK_MOTION_FIELDS if self.has_motion else ()):
             getattr(self, name)[s].zero_()
         for name, _ in K.TRACK_SCENE_FIELDS:
             getattr(self, name)[s] = 0
@@ -301,6 +317,31 @@ class TrackTable:
 def _to_device(values, dtype, dev):
     t = torch.tensor(values, dtype=dtype)
     return t.pin_memory().to(dev, non_blocking=True) if dev.type == "cuda" else t
+
+
+class MotionModel:
+    """The constant-velocity Kalman filter a ReIDTracker keeps per track (include/pcreid.h, pcreid_track_predict), with
+    AB3DMOT's settings as defaults.  State: the box (x, y, z, dx, dy, dz, yaw) and a velocity (vx, vy, vz) per unit of dt.
+      init_var      initial variance of the 7 box values            q      process noise of the box values, per step
+      init_vel_var  initial variance of the velocity                q_vel  process noise of the velocity, per step
+      r             measurement noise of each box value
+      gate_chi2     bound on the Mahalanobis distance of the predicted ground-plane centre to a detection's (chi-square,
+                    2 degrees of freedom: 9.21 is the 99 % quantile); None: no such bound"""
+
+    def __init__(self, init_var=10.0, init_vel_var=1e4, q=1.0, q_vel=0.01, r=1.0, gate_chi2=9.21):
+        positive = ("init_var", "init_vel_var", "r", "gate_chi2")
+        for name, v in dict(init_var=init_var, init_vel_var=init_vel_var, q=q, q_vel=q_vel, r=r, gate_chi2=gate_chi2).items():
+            if v is None and name == "gate_chi2":
+                setattr(self, name, None)
+                continue
+            v = float(v)
+            if not math.isfinite(v) or v < 0 or (v == 0 and name in positive):
+                raise ValueError(f"MotionModel.{name} must be finite and {'> 0' if name in positive else '>= 0'}; got {v}")
+            setattr(self, name, v)
+
+    def __repr__(self):
+        return (f"MotionModel(init_var={self.init_var}, init_vel_var={self.init_vel_var}, q={self.q}, q_vel={self.q_vel}, "
+                f"r={self.r}, gate_chi2={self.gate_chi2})")
 
 
 class ReIDTracker:
@@ -319,14 +360,24 @@ class ReIDTracker:
 
     With max_age=None, a capacity that never fills and no max_distance, slots are handed out in append order and scene s's
     table is, row for row, the bank of PointReidentifier.step called with track_index = arange(len(bank)) and the stored
-    labels; a detection's track id is then that bank row."""
+    labels; a detection's track id is then that bank row.
+
+    ``motion``: None or a MotionModel.  With a model, the table keeps a Kalman filter per slot and the step runs
+    kernels.track_predict (every active track of a scene with a frame, by that scene's ``dt``), then
+    kernels.track_gate_motion_blocks instead of track_gate_blocks (``max_distance`` around the predicted centre, plus
+    ``gate_chi2``), and kernels.track_correct after track_update (matched tracks take their detection, new tracks start with
+    velocity 0): two launches more and no further host read.  A frozen scene is not predicted; pass the time elapsed since its
+    last frame at its next one.  ``table.tracks(s)`` still gives the last matched boxes, ``table.motion(s)`` the filter's."""
 
     def __init__(self, model, num_scenes=1, capacity=1024, max_age=None, max_distance=None, replace_all=False, use_lengths=True,
-                 num_classes=8, min_points=2, subsample_number=128, device="cuda"):
+                 num_classes=8, min_points=2, subsample_number=128, device="cuda", motion=None):
         if max_age is not None and max_age < 0:
             raise ValueError("max_age must be None or >= 0")
+        if motion is not None and not isinstance(motion, MotionModel):
+            raise TypeError("motion must be None or a MotionModel")
         self.model = model
-        self.table = TrackTable(num_scenes, capacity, replace_all, device)
+        self.motion = motion
+        self.table = TrackTable(num_scenes, capacity, replace_all, device, motion=motion is not None)
         self.max_age, self.use_lengths = max_age, use_lengths
         self.num_classes, self.min_points, self.subsample_number = num_classes, min_points, subsample_number
         self.radius_sq = None
@@ -339,9 +390,10 @@ class ReIDTracker:
             self.radius_sq = (r * r).contiguous().to(self.table.device)
 
     @torch.no_grad()
-    def step(self, frames, min_score, sample_ranks=None):
+    def step(self, frames, min_score, sample_ranks=None, dt=1.0):
         """frames[s]: (sweep (P, >=3), bboxes (D_s, >=7), det_labels (D_s,)) or None (the scene is frozen: nothing ages);
-        sample_ranks: None (drawn on the device) or one (D_s, N) int64 tensor per scene with a frame.
+        sample_ranks: None (drawn on the device) or one (D_s, N) int64 tensor per scene with a frame; dt: with a motion model,
+        the time since each scene's previous frame, a float or one per scene (finite, >= 0; a frozen scene's entry is ignored).
         -> per scene (track_id_for_det (D_s,) int64, -1 for a detection that found no free slot; cost (A_s, D_s) logits, 0
         where not compared, or None when the scene had no active tracks), None for a frozen scene."""
         tab = self.table
@@ -354,6 +406,8 @@ class ReIDTracker:
             return results
         if sample_ranks is not None and any(sample_ranks[s] is None for s in live):
             raise ValueError("sample_ranks must give ranks for every scene with a frame, or be None")
+        if self.motion is not None:
+            dt = K.track_dt(dt, S, frozen=[s for s, f in enumerate(frames) if f is None])
         counts = tab.count.tolist()                                        # the step's one host read
         sweeps = [frames[s][0].float() for s in live]
         boxes = [frames[s][1][:, :7].float() for s in live]
@@ -374,9 +428,15 @@ class ReIDTracker:
         # 3. one gather of the rows of every scene's active tracks
         rows = tab.active.view(-1)[_to_device([s * C + i for s in range(S) for i in range(A[s])], torch.int64, dev)].long()
         xyz_t, h_t = tab.xyz[rows], tab.feat[rows]
-        # 4. the gate of every scene's (A_s, D_s) block
-        gate = K.track_gate_blocks(tab, shapes, det_label, det_length, det_box, self.num_classes, self.min_points,
-                                   self.use_lengths, self.radius_sq)
+        # 4. the gate of every scene's (A_s, D_s) block (with motion: on the predicted boxes)
+        mm = self.motion
+        if mm is None:
+            gate = K.track_gate_blocks(tab, shapes, det_label, det_length, det_box, self.num_classes, self.min_points,
+                                       self.use_lengths, self.radius_sq)
+        else:
+            K.track_predict(tab, shapes, dt, mm.q, mm.q_vel)
+            gate = K.track_gate_motion_blocks(tab, shapes, det_label, det_length, det_box, self.num_classes, self.min_points,
+                                              self.use_lengths, self.radius_sq, mm.r, mm.gate_chi2)
         d0, t0, e0 = [0], [0], [0]
         for a, d in shapes:
             d0.append(d0[-1] + d)
@@ -396,6 +456,8 @@ class ReIDTracker:
         _, track_for_det = K.linear_assignment_blocks(cost, shapes, min_score, gate)
         det_track_id, det_row = K.track_update(tab, shapes, track_for_det, det_label, det_length, det_box, self.max_age,
                                                tab.replace_all)
+        if mm is not None:
+            K.track_correct(tab, shapes, rows, track_for_det, det_box, det_row, mm.init_var, mm.init_vel_var, mm.r)
         K.track_scatter(det_row, xyz_d, h_d, tab.xyz, tab.feat)
         for s in live:
             results[s] = (det_track_id[d0[s]:d0[s + 1]], cost[e0[s]:e0[s + 1]].view(A[s], D[s]) if A[s] else None)

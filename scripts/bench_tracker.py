@@ -14,7 +14,14 @@ for launches): front_end, encode, score, assign, and for the bank / table work
   bank_update: PointFeatureSet.replace_old + store_new          | kernels.track_update + kernels.track_scatter
 and "outside" = step total - the sum of the phases.  Then the sequence once more with max_age=2 and a capacity of
 twice the largest D_s for the tracker (the banks of MultiScenePointReidentifier only grow): bank bytes after the last frame.  Writes a header line (GPU name, power limit and
-clocks read in the same run) and one JSON line per S to --out."""
+clocks read in the same run) and one JSON line per S to --out.
+
+--motion: instead, ReIDTracker with MotionModel() (AB3DMOT's defaults, dt = 1) against ReIDTracker without a motion model over
+the same sequence, alternated frame by frame, ids and alive tracks per frame compared; the phase pass adds "predict"
+(kernels.track_predict) and "correct" (kernels.track_correct), and "gate" covers kernels.track_gate_motion_blocks.  The boxes
+do not move, but the two trackers need not agree: without a bound a detection may match any track of its class, while the
+Mahalanobis bound leaves it only the tracks near its box, so a detection whose own track scores <= min_score starts a new
+track, and the step then scores more tracks."""
 import argparse
 import json
 import os
@@ -37,6 +44,11 @@ class TablePhaseTimer(PhaseTimer):
     PHASES = dict(PhaseTimer.PHASES, gate=[(TR, "class_gate"), (K, "track_gate_blocks")],
                   bank_update=[(TR.PointFeatureSet, "replace_old"), (TR.PointFeatureSet, "store_new"), (K, "track_update"),
                                (K, "track_scatter")])
+
+
+class MotionPhaseTimer(TablePhaseTimer):
+    PHASES = dict(TablePhaseTimer.PHASES, gate=TablePhaseTimer.PHASES["gate"] + [(K, "track_gate_motion_blocks")],
+                  predict=[(K, "track_predict")], correct=[(K, "track_correct")])
 
 
 def sequence(model, S, frames):
@@ -91,18 +103,62 @@ def timed_step(fn):
     return e0.elapsed_time(e1), out
 
 
+def motion_rows(model, a):
+    """--motion: one JSON line per S, the tracker with MotionModel() against the tracker without one"""
+    for S in [int(x) for x in a.scenes.split(",")]:
+        dets, ranks = sequence(model, S, a.frames)
+        capacity = min(K.TRACK_MAX_CAPACITY, a.frames * max(d[1].shape[0] for d in dets[0]))
+        make = {"plain": lambda: TR.ReIDTracker(model, num_scenes=S, capacity=capacity),
+                "motion": lambda: TR.ReIDTracker(model, num_scenes=S, capacity=capacity, motion=TR.MotionModel())}
+        # timed pass, alternated frame by frame; ids compared
+        trackers = {k: f() for k, f in make.items()}
+        times, identical, alive = {k: [] for k in make}, True, {k: [] for k in make}
+        for f in range(a.frames):
+            out = {}
+            for k, tr in trackers.items():
+                t, out[k] = timed_step(lambda: tr.step(dets[f], MIN_SCORE, sample_ranks=ranks[f], dt=1.0))
+                alive[k].append(int(tr.table.count.sum()))
+                if f >= a.warmup:
+                    times[k].append(t)
+            identical &= all(torch.equal(x[0], y[0]) for x, y in zip(out["plain"], out["motion"]))
+        # phase pass
+        phases = {}
+        for k, f_make in make.items():
+            tr, per = f_make(), []
+            for f in range(a.frames):
+                with MotionPhaseTimer(model) as pt:
+                    total, _ = timed_step(lambda: tr.step(dets[f], MIN_SCORE, sample_ranks=ranks[f], dt=1.0))
+                p = pt.totals()
+                p["outside"] = total - sum(p.values())
+                p["step"] = total
+                if f >= a.warmup:
+                    per.append(p)
+            phases[k] = {n: round(statistics.median(p[n] for p in per), 3) for n in per[0]}
+        del trackers, tr
+        med = {k: statistics.median(v) for k, v in times.items()}
+        yield {"S": S, "detections_per_frame": sum(d[1].shape[0] for d in dets[0]), "capacity": capacity,
+               "identical_ids": bool(identical), "alive_tracks_per_frame": alive, "plain_ms": round(med["plain"], 3), "motion_ms": round(med["motion"], 3),
+               "motion_minus_plain_ms": round(med["motion"] - med["plain"], 3),
+               "plain_ms_all": [round(t, 3) for t in times["plain"]], "motion_ms_all": [round(t, 3) for t in times["motion"]],
+               "phases_ms": phases}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--scenes", default="1,8,32,128")
     ap.add_argument("--frames", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=2)
+    ap.add_argument("--motion", action="store_true", help="the tracker with a motion model against the tracker without")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     model, _ = helpers.build_pair("pt", (128, 64, 32), device=DEV)
     model.set_mode("parity_tc")
     lines = [dict(gpu_header(), frames=a.frames)]
     print(json.dumps(lines[0]), flush=True)
-    for S in [int(x) for x in a.scenes.split(",")]:
+    for row in (motion_rows(model, a) if a.motion else ()):
+        lines.append(row)
+        print(json.dumps(row), flush=True)
+    for S in ([] if a.motion else [int(x) for x in a.scenes.split(",")]):
         dets, ranks = sequence(model, S, a.frames)
         capacity = min(K.TRACK_MAX_CAPACITY, a.frames * max(d[1].shape[0] for d in dets[0]))
         # timed pass, alternated frame by frame; outputs compared
